@@ -91,6 +91,27 @@ def workload_string(name, flat):
             f"brute force over every primitive")
 
 
+DUMP_LIMIT_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, images):
+    """Writes each [ny, nx, c] image as out_dir/<name>.npy, keeping its dtype (float32 or float64).  When all of them
+    together pass 64 MB, every image keeps the same fixed, seeded sample of pixels instead: [k, c] in increasing pixel
+    order (row-major over [ny, nx]), and pixel_index.npy (float64) holds those k flat pixel indices.  The device adds
+    float samples in a varying order, so two runs agree to the last bits of the sums (and 1 of 255 in rgb8), not exactly."""
+    os.makedirs(out_dir, exist_ok=True)
+    ny, nx = next(iter(images.values())).shape[:2]
+    n_pix = ny * nx
+    bytes_per_pix = sum(a.shape[2] * a.itemsize for a in images.values())
+    if n_pix * bytes_per_pix > DUMP_LIMIT_BYTES:
+        k = (DUMP_LIMIT_BYTES - 4096) // (bytes_per_pix + 8)       # 4 KiB left for the .npy headers
+        idx = np.sort(np.random.default_rng(0).choice(n_pix, k, replace=False))
+        images = {name: a.reshape(n_pix, a.shape[2])[idx] for name, a in images.items()}
+        np.save(os.path.join(out_dir, "pixel_index.npy"), idx.astype(np.float64))
+    for name, a in images.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
+
+
 def host_cores():
     try:
         return len(os.sched_getaffinity(0))
@@ -171,10 +192,13 @@ def run_reference(args, world, rank):
     t0 = time.perf_counter()
     samples = tests = 0
     for k in range(args.steps):
-        _, c = S.render_accumulate(cam_type, cam, nx, ny, (k * step_spp) % max(1, spp), step_spp, depth, seed=1 + k, n_threads=cores)
+        sum_rgb, c = S.render_accumulate(cam_type, cam, nx, ny, (k * step_spp) % max(1, spp), step_spp, depth, seed=1 + k, n_threads=cores)
         samples += c["samples"]
         tests += c["sphere_tests"]
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        # the last step's float sums over its samples (row 0 = bottom) and the 8-bit frame they resolve to (row 0 = top)
+        dump_outputs(args.dump_outputs, {"linear_sum": sum_rgb, "rgb8": oracle.resolve(sum_rgb, step_spp).astype(np.float64)})
     v = samples / dt
     sample = f"{nx}x{ny}, {step_spp} of {spp} spp per step, depth {depth}, brute force over {flat.n_spheres} primitives, double precision"
     line = {
@@ -246,7 +270,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-strong-c3", action="store_true", help="skip the BASELINE config 3 strong-scaling block")
     ap.add_argument("--e2e-steps", type=int, default=0, help="default: min(steps, 10)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy: linear_sum (the float "
+                         "sums over its samples) and rgb8 (the resolved frame, as floats); inputs depend only on the arguments. "
+                         "bench_outputs/ in the repository is git-ignored for this")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -341,6 +371,9 @@ def main():
         ev[k][1].record(stream)
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # the last timed step's float sums over all its samples (row 0 = bottom) and the 8-bit frame (row 0 = top)
+        dump_outputs(args.dump_outputs, {"linear_sum": d_sum.cpu().numpy(), "rgb8": d_rgb.cpu().numpy().astype(np.float32)})
     my_ms = sum(a.elapsed_time(b) for a, b in ev)
     my_kernel_ms = sum(a.elapsed_time(b) for a, b in kev)
     ctr = r.counters()
