@@ -225,7 +225,9 @@ int rt_set_accel(rt_ctx* ctx, int accel);
  * cores whatever the list length),
  * "tc_tiles_per_cta", "tc_ctas", "wave_depth", "tail_rays", "tail_solo" (a tail slice of this many paths or fewer runs one warp per
  * path, default 24; 0 = staged to the end), "tail_lpp" (lanes per such path: 8 | 16 | 32), "tail_block", "cull_shape",
- * "tail_ctas_per_sm", "mega_regcap".
+ * "tail_ctas_per_sm", "mega_regcap", "bvh_build" (where RT_ACCEL_BVH's tree is built: 1 = on the device from 1000 listed leaves
+ * up, on the host below (default), 0 = host always, 2 = device always; a device tree deeper than the traversal's 48-entry
+ * stack is replaced by the host build before any ray sees it).
  * Unknown name -> RT_ERR_ARG.                                                                                     */
 int rt_set_option(rt_ctx* ctx, const char* name, int64_t value);
 int rt_set_camera(rt_ctx* ctx, int cam_type, const float cam[24]);
@@ -250,6 +252,14 @@ int rt_render(rt_ctx* ctx, int nx, int ny, int nsamples, int max_depth, uint64_t
  * ByteBuffer.  ctx may be NULL (the memory is usable with every context of the process).        */
 int rt_host_alloc(rt_ctx* ctx, size_t bytes, void** out);
 int rt_host_free(rt_ctx* ctx, void* p);
+
+/* The RT_ACCEL_BVH tree as device `device_index` of the context holds it (built first if the scene or the movers' time
+ * window changed since the last build, whatever the accelerator): 16 floats per node (left child's box lo.xyz hi.xyz,
+ * right child's box lo.xyz hi.xyz, then left, right, 0, 0 as int32; a leaf child k in cull order is stored as ~k; the root is
+ * node 0).  out_nodes may be NULL; otherwise cap_nodes must be at least the node count.  info = {node count, depth of the
+ * deepest leaf (root = 0), builder (0 host, 1 device), device build time in ns from CUDA events (0 for the host build)}.
+ * Added within ABI version 2, like rt_host_alloc / rt_host_free.                                                        */
+int rt_get_bvh(rt_ctx* ctx, int device_index, float* out_nodes, int64_t cap_nodes, int64_t info[4]);
 
 /* Same render, device-resident: accumulate samples [sample_begin, sample_begin+sample_count)
  * of every pixel whose row j satisfies j % row_stride == row_offset into d_sum (DEVICE pointer on

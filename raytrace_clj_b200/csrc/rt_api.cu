@@ -21,6 +21,7 @@
 #include <string>
 #include <vector>
 
+#include "rt_bvh_build.cuh"
 #include "rt_kernels.cuh"
 
 using namespace rt;
@@ -83,6 +84,12 @@ struct DeviceBuffers {
     // RT_ACCEL_BVH: the flattened tree (4 float4 per node), rebuilt with the scene / the movers' time window
     float4* bvh_nodes = nullptr;
     size_t bvh_cap = 0;
+    int bvh_builder = 0, bvh_depth = 0;   // the published tree: 0 host / 1 device builder, depth of its deepest leaf
+    long long bvh_build_ns = 0;           // device build: CUDA-event time of the last one (upload included)
+    void* bvh_scratch = nullptr;          // device build: inputs, leaf boxes, codes, parents, flags, sort storage (grown on demand)
+    size_t bvh_scratch_bytes = 0;
+    int* h_bvh_depth = nullptr;           // pinned: the built tree's depth, read back before the tree is published
+    cudaEvent_t ev_b0 = nullptr, ev_b1 = nullptr;
     // pinned staging for the results of rt_render (root device): D2H at link speed, then one host memcpy into the caller's buffer
     void* h_stage = nullptr;
     size_t h_stage_bytes = 0;
@@ -130,6 +137,8 @@ struct Options {
                                       //   2 = except a lane's first, all-camera-ray iteration when those rays share an origin
     int tc_tiles_per_cta = 0;         // RT_TC_TILES_PER_CTA: ray tiles a wf_cull_tc CTA takes before it retires (0 = one CTA per SM, persistent)
     int tc_ctas = 0;                  // RT_TC_CTAS: persistent wf_cull_tc CTAs (0 = one per SM); fewer leaves whole SMs to the other lane's stage kernels
+    int bvh_build = 1;                // RT_BVH_BUILD: RT_ACCEL_BVH's tree built on the host (0), on the device (2), or on the device
+                                      //   from kBvhDeviceMinLeaves listed leaves up (1)
 };
 
 struct rt_ctx {
@@ -320,6 +329,7 @@ Options options_from_env() {
     o.cull_tc = env_int("RT_CULL_TC", o.cull_tc);
     o.tc_tiles_per_cta = env_int("RT_TC_TILES_PER_CTA", o.tc_tiles_per_cta);
     o.tc_ctas = env_int("RT_TC_CTAS", o.tc_ctas);
+    o.bvh_build = env_int("RT_BVH_BUILD", o.bvh_build);
     return o;
 }
 
@@ -827,9 +837,11 @@ struct BuildLeaf {
     float c[3];
     int k;
 };
-int bvh_build_node(std::vector<BuildLeaf>& L, int begin, int end, std::vector<float>& nodes, float lo[3], float hi[3]) {
+int bvh_build_node(std::vector<BuildLeaf>& L, int begin, int end, std::vector<float>& nodes, float lo[3], float hi[3], int depth,
+                   int* max_depth) {
     if (end - begin == 1) {
         for (int a = 0; a < 3; ++a) { lo[a] = L[(size_t)begin].lo[a]; hi[a] = L[(size_t)begin].hi[a]; }
+        *max_depth = std::max(*max_depth, depth);
         return ~L[(size_t)begin].k;
     }
     float cmin[3] = {INFINITY, INFINITY, INFINITY}, cmax[3] = {-INFINITY, -INFINITY, -INFINITY};
@@ -843,8 +855,8 @@ int bvh_build_node(std::vector<BuildLeaf>& L, int begin, int end, std::vector<fl
     const size_t me = nodes.size() / 16;
     nodes.resize(nodes.size() + 16, 0.f);
     float llo[3], lhi[3], rlo[3], rhi[3];
-    const int left = bvh_build_node(L, begin, mid, nodes, llo, lhi);
-    const int right = bvh_build_node(L, mid, end, nodes, rlo, rhi);
+    const int left = bvh_build_node(L, begin, mid, nodes, llo, lhi, depth + 1, max_depth);
+    const int right = bvh_build_node(L, mid, end, nodes, rlo, rhi, depth + 1, max_depth);
     float* N = nodes.data() + 16 * me;
     N[0] = llo[0]; N[1] = llo[1]; N[2] = llo[2]; N[3] = lhi[0]; N[4] = lhi[1]; N[5] = lhi[2];
     N[6] = rlo[0]; N[7] = rlo[1]; N[8] = rlo[2]; N[9] = rhi[0]; N[10] = rhi[1]; N[11] = rhi[2];
@@ -853,8 +865,18 @@ int bvh_build_node(std::vector<BuildLeaf>& L, int begin, int end, std::vector<fl
     for (int a = 0; a < 3; ++a) { lo[a] = std::min(llo[a], rlo[a]); hi[a] = std::max(lhi[a], rhi[a]); }
     return (int)me;
 }
-int ensure_bvh(rt_ctx* ctx) {
-    if (!ctx->bvh_dirty) return RT_OK;
+
+int ensure_bvh_nodes(rt_ctx* ctx, DeviceBuffers& d, size_t bytes) {
+    if (d.bvh_cap >= bytes) return RT_OK;
+    if (d.bvh_nodes) cudaFree(d.bvh_nodes);
+    d.bvh_nodes = nullptr;
+    d.bvh_cap = 0;
+    RT_CUDA(ctx, cudaMalloc(&d.bvh_nodes, bytes));
+    d.bvh_cap = bytes;
+    return RT_OK;
+}
+
+int bvh_build_host(rt_ctx* ctx) {
     const int n = ctx->n_list;
     std::vector<BuildLeaf> L((size_t)n);
     for (int k = 0; k < n; ++k) {
@@ -881,6 +903,7 @@ int ensure_bvh(rt_ctx* ctx) {
     std::vector<float> nodes;
     nodes.reserve(16 * (size_t)std::max(1, n));
     float lo[3], hi[3];
+    int depth = 1;
     if (n == 1) {   // a lone leaf is both children of the root (hitable.clj:113-114)
         nodes.assign(16, 0.f);
         for (int a = 0; a < 3; ++a) { nodes[(size_t)a] = nodes[6 + (size_t)a] = L[0].lo[a]; nodes[3 + (size_t)a] = nodes[9 + (size_t)a] = L[0].hi[a]; }
@@ -888,25 +911,126 @@ int ensure_bvh(rt_ctx* ctx) {
         memcpy(&nodes[12], &leaf, 4);
         memcpy(&nodes[13], &leaf, 4);
     } else {
-        const int root = bvh_build_node(L, 0, n, nodes, lo, hi);
+        const int root = bvh_build_node(L, 0, n, nodes, lo, hi, 0, &depth);
         if (root != 0) return fail(ctx, RT_ERR_STATE, "BVH build: the root is not node 0");
     }
     for (auto& d : ctx->devs) {
         RT_CUDA(ctx, cudaSetDevice(d.dev));
         RT_CUDA(ctx, cudaDeviceSynchronize());
         const size_t bytes = nodes.size() * sizeof(float);
-        if (d.bvh_cap < bytes) {
-            if (d.bvh_nodes) cudaFree(d.bvh_nodes);
-            d.bvh_nodes = nullptr;
-            d.bvh_cap = 0;
-            RT_CUDA(ctx, cudaMalloc(&d.bvh_nodes, bytes));
-            d.bvh_cap = bytes;
-        }
+        if (int rc = ensure_bvh_nodes(ctx, d, bytes)) return rc;
         RT_CUDA(ctx, cudaMemcpy(d.bvh_nodes, nodes.data(), bytes, cudaMemcpyHostToDevice));
         d.sc.bvh = d.bvh_nodes;
         d.sc.bvh_nodes = (int)(nodes.size() / 16);
+        d.bvh_builder = 0;
+        d.bvh_depth = depth;
+        d.bvh_build_ns = 0;
     }
     cudaSetDevice(ctx->devs[0].dev);
+    return RT_OK;
+}
+
+// RT_ACCEL_BVH on the device (rt_bvh_build.cuh): enqueue the whole build on one device's stream, the depth read back into
+// pinned memory last.  The tree lands in the node buffer; it is published (or replaced by the host build, when too deep)
+// after the stream has finished.
+int bvh_enqueue_device(rt_ctx* ctx, DeviceBuffers& d) {
+    const int n = ctx->n_list;
+    const int n_nodes = std::max(1, n - 1);
+    RT_CUDA(ctx, cudaSetDevice(d.dev));
+    RT_CUDA(ctx, cudaDeviceSynchronize());   // a render enqueued with sync = 0 on a caller's stream may still read the tree
+    if (int rc = ensure_bvh_nodes(ctx, d, (size_t)n_nodes * 4 * sizeof(float4))) return rc;
+    size_t sort_bytes = 0;
+    RT_CUDA(ctx, cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, (const unsigned long long*)nullptr, (unsigned long long*)nullptr,
+                                                 (const int*)nullptr, (int*)nullptr, n, 0, 3 * (int)kMortonAxisBits, d.stream));
+    size_t off = 0;
+    auto take = [&](size_t bytes) { const size_t o = off; off = align_up(off + bytes, 256); return o; };
+    const size_t n_ = (size_t)n;
+    const size_t o_c0 = take(n_ * 3 * 8), o_c1 = take(n_ * 3 * 8), o_r = take(n_ * 8), o_t = take(n_ * 2 * 4), o_fl = take(n_ * 4);
+    const size_t o_box = take(n_ * 6 * 4), o_cb = take(6 * 4), o_code = take(n_ * 8), o_code2 = take(n_ * 8);
+    const size_t o_leaf = take(n_ * 4), o_leaf2 = take(n_ * 4), o_par = take((2 * n_ - 1) * 4), o_arr = take((size_t)n_nodes * 4);
+    const size_t o_h = take((size_t)n_nodes * 4), o_depth = take(4), o_sort = take(sort_bytes);
+    if (d.bvh_scratch_bytes < off) {
+        if (d.bvh_scratch) cudaFree(d.bvh_scratch);
+        d.bvh_scratch = nullptr;
+        d.bvh_scratch_bytes = 0;
+        RT_CUDA(ctx, cudaMalloc(&d.bvh_scratch, off));
+        d.bvh_scratch_bytes = off;
+    }
+    if (!d.h_bvh_depth) {
+        RT_CUDA(ctx, cudaHostAlloc(&d.h_bvh_depth, sizeof(int), cudaHostAllocDefault));
+        RT_CUDA(ctx, cudaEventCreate(&d.ev_b0));
+        RT_CUDA(ctx, cudaEventCreate(&d.ev_b1));
+    }
+    char* S = (char*)d.bvh_scratch;
+    const cudaStream_t st = d.stream;
+    BvhLeafInput in{(const double*)(S + o_c0), (const double*)(S + o_c1), (const double*)(S + o_r), (const float*)(S + o_t),
+                    (const unsigned*)(S + o_fl)};
+    float* boxes = (float*)(S + o_box);
+    unsigned* cb = (unsigned*)(S + o_cb);
+    int* depth = (int*)(S + o_depth);
+    RT_CUDA(ctx, cudaEventRecord(d.ev_b0, st));
+    RT_CUDA(ctx, cudaMemcpyAsync(S + o_c0, ctx->h_bs_c0.data(), n_ * 3 * 8, cudaMemcpyHostToDevice, st));
+    RT_CUDA(ctx, cudaMemcpyAsync(S + o_c1, ctx->h_bs_c1.data(), n_ * 3 * 8, cudaMemcpyHostToDevice, st));
+    RT_CUDA(ctx, cudaMemcpyAsync(S + o_r, ctx->h_bs_r.data(), n_ * 8, cudaMemcpyHostToDevice, st));
+    RT_CUDA(ctx, cudaMemcpyAsync(S + o_t, ctx->h_t0t1.data(), n_ * 2 * 4, cudaMemcpyHostToDevice, st));
+    RT_CUDA(ctx, cudaMemcpyAsync(S + o_fl, ctx->h_flags.data(), n_ * 4, cudaMemcpyHostToDevice, st));
+    RT_CUDA(ctx, cudaMemsetAsync(cb, 0xff, 3 * 4, st));   // min of the centroids: from the largest key
+    RT_CUDA(ctx, cudaMemsetAsync(cb + 3, 0, 3 * 4, st));  // max: from the smallest
+    const int grid = (n + 255) / 256;
+    bvh_leaf_boxes<<<grid, 256, 0, st>>>(in, n, ctx->win_lo, ctx->win_hi, boxes, cb);
+    if (n == 1) {
+        bvh_single_leaf<<<1, 32, 0, st>>>(boxes, d.bvh_nodes, depth);
+    } else {
+        unsigned long long* code = (unsigned long long*)(S + o_code);
+        unsigned long long* code2 = (unsigned long long*)(S + o_code2);
+        int* leaf = (int*)(S + o_leaf);
+        int* leaf2 = (int*)(S + o_leaf2);
+        int* parent = (int*)(S + o_par);
+        bvh_morton<<<grid, 256, 0, st>>>(boxes, n, cb, code, leaf);
+        RT_CUDA(ctx, cub::DeviceRadixSort::SortPairs(S + o_sort, sort_bytes, code, code2, leaf, leaf2, n, 0, 3 * (int)kMortonAxisBits, st));
+        RT_CUDA(ctx, cudaMemsetAsync(S + o_arr, 0, (size_t)n_nodes * 4, st));
+        bvh_hierarchy<<<(n - 1 + 255) / 256, 256, 0, st>>>(code2, leaf2, n, d.bvh_nodes, parent);
+        bvh_fit<<<grid, 256, 0, st>>>(boxes, parent, n, d.bvh_nodes, (unsigned*)(S + o_arr), (int*)(S + o_h), depth);
+    }
+    RT_CUDA(ctx, cudaGetLastError());
+    RT_CUDA(ctx, cudaMemcpyAsync(d.h_bvh_depth, depth, sizeof(int), cudaMemcpyDeviceToHost, st));
+    RT_CUDA(ctx, cudaEventRecord(d.ev_b1, st));
+    d.sc.bvh_nodes = n_nodes;
+    return RT_OK;
+}
+
+// Listed leaves from which the automatic choice (option bvh_build = 1) builds the tree on the device.  Measured on a B200
+// (profiles/r03_bvh_build.txt, DESIGN §7): from 1 003 leaves up the device tree gives the shorter time to image (C5 shape,
+// 1 k - 1 M leaves: its build is shorter and its frames too); on C2's 485 leaves the host tree renders 0.6 ms faster while
+// either build takes 0.1 ms.
+constexpr int kBvhDeviceMinLeaves = 1000;
+
+// RT_ACCEL_BVH: (re)build the tree when the scene or the movers' window changed.  The device build runs on every device
+// of the context at once; a tree deeper than bvh_closest's stack allows is never published — the host build (median
+// splits, depth ~log2 n) replaces it.
+int ensure_bvh(rt_ctx* ctx) {
+    if (!ctx->bvh_dirty) return RT_OK;
+    const int mode = ctx->opt.bvh_build;
+    const bool on_device = mode == 2 || (mode == 1 && ctx->n_list >= kBvhDeviceMinLeaves);
+    bool too_deep = false;
+    if (on_device) {
+        for (auto& d : ctx->devs)
+            if (int rc = bvh_enqueue_device(ctx, d)) return rc;
+        for (auto& d : ctx->devs) {
+            RT_CUDA(ctx, cudaSetDevice(d.dev));
+            RT_CUDA(ctx, cudaStreamSynchronize(d.stream));
+            float ms = 0.f;
+            RT_CUDA(ctx, cudaEventElapsedTime(&ms, d.ev_b0, d.ev_b1));
+            d.sc.bvh = d.bvh_nodes;
+            d.bvh_builder = 1;
+            d.bvh_depth = *d.h_bvh_depth;
+            d.bvh_build_ns = (long long)((double)ms * 1e6);
+            too_deep |= d.bvh_depth > kBvhMaxDepth;
+        }
+        cudaSetDevice(ctx->devs[0].dev);
+    }
+    if (!on_device || too_deep)
+        if (int rc = bvh_build_host(ctx)) return rc;
     ctx->bvh_dirty = false;
     return RT_OK;
 }
@@ -1058,6 +1182,10 @@ void rt_destroy(rt_ctx* ctx) {
         for (auto& e : d.ev_chunk) if (e) cudaEventDestroy(e);
         if (d.h_stage) cudaFreeHost(d.h_stage);
         if (d.bvh_nodes) cudaFree(d.bvh_nodes);
+        if (d.bvh_scratch) cudaFree(d.bvh_scratch);
+        if (d.h_bvh_depth) cudaFreeHost(d.h_bvh_depth);
+        if (d.ev_b0) cudaEventDestroy(d.ev_b0);
+        if (d.ev_b1) cudaEventDestroy(d.ev_b1);
         if (d.stream) cudaStreamDestroy(d.stream);
     }
     delete ctx;
@@ -1505,6 +1633,29 @@ int rt_set_accel(rt_ctx* ctx, int accel) {
     return RT_OK;
 }
 
+int rt_get_bvh(rt_ctx* ctx, int device_index, float* out_nodes, int64_t cap_nodes, int64_t info[4]) {
+    if (!ctx) return RT_ERR_ARG;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    if (int rc = check_ready(ctx)) return rc;
+    if (device_index < 0 || device_index >= (int)ctx->devs.size()) return fail(ctx, RT_ERR_ARG, "device_index out of range");
+    if (int rc = ensure_bvh(ctx)) return rc;
+    DeviceBuffers& d = ctx->devs[(size_t)device_index];
+    const int64_t n_nodes = d.sc.bvh_nodes;
+    if (info) {
+        info[0] = n_nodes;
+        info[1] = d.bvh_depth;
+        info[2] = d.bvh_builder;
+        info[3] = d.bvh_build_ns;
+    }
+    if (out_nodes) {
+        if (cap_nodes < n_nodes) return fail(ctx, RT_ERR_ARG, "cap_nodes is below the node count (info[0])");
+        RT_CUDA(ctx, cudaSetDevice(d.dev));
+        RT_CUDA(ctx, cudaMemcpy(out_nodes, d.bvh_nodes, (size_t)n_nodes * 4 * sizeof(float4), cudaMemcpyDeviceToHost));
+        cudaSetDevice(ctx->devs[0].dev);
+    }
+    return RT_OK;
+}
+
 int rt_set_option(rt_ctx* ctx, const char* name, int64_t value) {
     if (!ctx) return RT_ERR_ARG;
     std::lock_guard<std::mutex> lk(ctx->mu);
@@ -1533,6 +1684,7 @@ int rt_set_option(rt_ctx* ctx, const char* name, int64_t value) {
     else if (k == "cull_tc") o.cull_tc = (int)value;
     else if (k == "tc_tiles_per_cta") o.tc_tiles_per_cta = (int)value;
     else if (k == "tc_ctas") o.tc_ctas = (int)value;
+    else if (k == "bvh_build") o.bvh_build = (int)value;   // takes effect at the next tree build
     else return fail(ctx, RT_ERR_ARG, "unknown option: " + k);
     return RT_OK;
 }

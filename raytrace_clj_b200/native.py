@@ -380,6 +380,7 @@ ABI_SYMBOLS = [
     "rt_render_accumulate_device", "rt_resolve_device", "rt_trace_primary", "rt_generate_rays", "rt_shade_batch",
     "rt_measure_fp32_peak", "rt_get_counters", "rt_reset_counters", "rt_set_profile", "rt_device_info", "rt_cull_check",
     "rt_set_scene_ex", "rt_trace_paths", "rt_set_accel", "rt_set_option", "rt_sample_device", "rt_host_alloc", "rt_host_free",
+    "rt_get_bvh",
 ]
 
 _lib = None
@@ -425,6 +426,7 @@ def load_library():
     L.rt_device_info.argtypes = [C.c_void_p, _i32p, _i32p, C.c_char_p]
     L.rt_host_alloc.argtypes = [C.c_void_p, C.c_size_t, C.POINTER(C.c_void_p)]
     L.rt_host_free.argtypes = [C.c_void_p, C.c_void_p]
+    L.rt_get_bvh.argtypes = [C.c_void_p, C.c_int, _f32p, C.c_int64, C.POINTER(C.c_int64)]
     _lib = L
     return L
 
@@ -536,6 +538,18 @@ class Renderer:
     def set_accel(self, accel):
         """RT_ACCEL_BRUTE_FORCE (the roofline path) or RT_ACCEL_BVH (flattened GPU BVH, hitable.clj:97-123's role)."""
         self._check(self.L.rt_set_accel(self.h, int(accel)), "rt_set_accel")
+
+    def bvh(self, device_index=0):
+        """rt_get_bvh: the RT_ACCEL_BVH tree of one device of the context (built first if it is out of date).  Returns
+        (nodes [count, 16] f32 — words 12..15 hold int32 (left, right, 0, 0), a leaf child k as ~k — and
+        {"nodes", "depth", "builder" ("host" | "device"), "build_ns"})."""
+        info = np.zeros(4, np.int64)
+        ip = info.ctypes.data_as(C.POINTER(C.c_int64))
+        self._check(self.L.rt_get_bvh(self.h, int(device_index), None, 0, ip), "rt_get_bvh")
+        nodes = np.zeros((int(info[0]), 16), np.float32)
+        self._check(self.L.rt_get_bvh(self.h, int(device_index), _p(nodes, _f32p), int(info[0]), ip), "rt_get_bvh")
+        return nodes, {"nodes": int(info[0]), "depth": int(info[1]), "builder": ("host", "device")[int(info[2])],
+                       "build_ns": int(info[3])}
 
     def set_option(self, name, value):
         """Per-context tuning knob (the RT_* environment variables are only the defaults)."""
