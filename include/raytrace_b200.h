@@ -215,6 +215,21 @@ int rt_abi_version(void);
 int rt_set_scene(rt_ctx* ctx, const rt_scene_desc* scene);
 /* the same with the extension record (ext may be NULL = rt_set_scene) */
 int rt_set_scene_ex(rt_ctx* ctx, const rt_scene_desc* scene, const rt_scene_ext* ext);
+/* rt_set_scene for a scene whose PER-PRIMITIVE arrays live in device memory on the context's first device:
+ * center0_r, center1, t0t1, sphere_flags, material_id are DEVICE pointers (center1 / t0t1 / sphere_flags may be NULL as
+ * in rt_set_scene); the material and texture tables stay HOST pointers.  Spheres / UVSpheres / MovingSpheres with the
+ * four rt_set_scene materials and three textures only (everything rt_set_scene accepts; nothing of rt_scene_ext).
+ * The library orders its reads after the work already enqueued on `stream` (a cudaStream_t, NULL = legacy default);
+ * it returns once the scene is built, so the caller may overwrite or free the arrays afterwards.
+ * Same validation, status codes and messages as rt_set_scene; a rejected scene leaves the previous one in place.
+ * The scene then behaves exactly as if rt_set_scene had been given the same values: the GPU builds the same blob bytes
+ * (the host's marshalling restated kernel by kernel), so a caller whose spheres are already on the GPU (a simulation, a
+ * generated scene) skips the copy to the host, the single-threaded marshalling and the upload.  A per-primitive pointer
+ * that is not device or managed memory of device_ids[0] -> RT_ERR_ARG.  Added within ABI version 2, like rt_get_bvh. */
+int rt_set_scene_device(rt_ctx* ctx, const rt_scene_desc* scene, void* stream);
+/* The scene blob device `device_index` holds (diagnostic): out may be NULL to query *bytes; otherwise cap >= *bytes.
+ * Added within ABI version 2.                                                                                       */
+int rt_get_scene_blob(rt_ctx* ctx, int device_index, void* out, size_t cap, size_t* bytes);
 /* closest-hit search used by the renders that follow: RT_ACCEL_BRUTE_FORCE (default) or RT_ACCEL_BVH */
 int rt_set_accel(rt_ctx* ctx, int accel);
 /* Per-context tuning knob; the RT_* environment variables only give the defaults at rt_create.  Names:

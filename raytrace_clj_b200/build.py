@@ -9,7 +9,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libraytrace_b200.so")
 SOURCES = ["rt_api.cu"]
-HEADERS = ["rt_device.cuh", "rt_kernels.cuh", "rt_cull_tc.cuh", "rt_bvh_build.cuh", os.path.join("..", "..", "include", "raytrace_b200.h")]
+HEADERS = ["rt_device.cuh", "rt_kernels.cuh", "rt_cull_tc.cuh", "rt_bvh_build.cuh", "rt_scene_build.cuh", os.path.join("..", "..", "include", "raytrace_b200.h")]
 
 NVCC_FLAGS = (["-DRT_TAIL_DIAG"] if os.environ.get("RT_TAIL_DIAG") else []) + [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",

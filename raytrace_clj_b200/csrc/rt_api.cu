@@ -23,6 +23,7 @@
 
 #include "rt_bvh_build.cuh"
 #include "rt_kernels.cuh"
+#include "rt_scene_build.cuh"
 
 using namespace rt;
 
@@ -44,6 +45,16 @@ struct DeviceBuffers {
     void* scene_blob = nullptr;
     void* scene_stage = nullptr;
     size_t scene_bytes = 0;
+    size_t scene_used = 0;                // bytes of the current scene's blob
+    // rt_set_scene_device: the listed leaves' FP64 bounding spheres stay on the device (c0, c1, r; t0t1 and flags are the
+    // blob's), in the layout the device BVH build reads
+    void* bs_buf = nullptr;
+    size_t bs_bytes = 0;
+    BvhLeafInput bs_in{};
+    void* sb_scratch = nullptr;           // device 0: radii, sort storage, candidates, cull order of the device build
+    size_t sb_scratch_bytes = 0;
+    SbResult* h_sb = nullptr;             // pinned: the validation / direct-sphere result read back before the blob is laid out
+    cudaEvent_t ev_sb = nullptr;          // orders the build after the caller's stream
     DevScene sc{};
     // frame
     float* d_sum = nullptr;
@@ -164,6 +175,10 @@ struct rt_ctx {
     std::vector<unsigned> h_flags;
     // world-space bounding sphere of every world leaf, cull order: centre at t0 / t1 (equal unless moving), radius
     std::vector<double> h_bs_c0, h_bs_c1, h_bs_r;
+    // rt_set_scene_device: the bounding spheres live on every device (DeviceBuffers::bs_in); h_bs_*, h_t0t1 and h_flags are
+    // a mirror downloaded on demand (bs_mirror), and tc_row_k / tc_scratch_rows are unused (the rows are in the blob)
+    bool bs_on_device = false, bs_mirror = false;
+    bool any_moving = false;      // some listed or direct sphere moves (rt_set_scene_device)
     DevCamera cam{};
     std::atomic<uint64_t> n_launches{0};
     std::mutex err_mu;
@@ -804,12 +819,40 @@ void build_cull_records(rt_ctx* ctx, double win_lo, double win_hi, float* cull_a
     }
 }
 
+// build_cull_records on one device over its device-resident bounding spheres (a scene of rt_set_scene_device): the FP32
+// records, the padding records and the tensor-core feature rows of the rows the blob's tc_row_k deals out
+int enqueue_records_device(rt_ctx* ctx, DeviceBuffers& d, double win_lo, double win_hi) {
+    const int n = ctx->n_spheres, pad = ctx->n_cull - ctx->n_list, rows = ctx->tc_tiles * tc::TILE_N;
+    sb_cull_records<<<(n + pad + kSbBlock - 1) / kSbBlock, kSbBlock, 0, d.stream>>>(d.bs_in, n, ctx->n_list, ctx->n_cull, win_lo, win_hi,
+                                                                                    const_cast<float4*>(d.sc.cull_a));
+    if (rows)
+        sb_tc_rows<<<(rows + kSbBlock - 1) / kSbBlock, kSbBlock, 0, d.stream>>>(d.bs_in, d.sc.tc_row_k, rows, win_lo, win_hi,
+                                                                                const_cast<float*>(d.sc.cull_tc));
+    RT_CUDA(ctx, cudaGetLastError());
+    return RT_OK;
+}
+
 // make sure the movers' bounding spheres cover ray times in [lo, hi]
 int ensure_window(rt_ctx* ctx, double lo, double hi) {
     if (lo >= ctx->win_lo && hi <= ctx->win_hi) return RT_OK;
     if (!(lo <= hi) || !std::isfinite(lo) || !std::isfinite(hi)) return fail(ctx, RT_ERR_ARG, "ray time is not finite");
     ctx->win_lo = std::min(ctx->win_lo, lo);
     ctx->win_hi = std::max(ctx->win_hi, hi);
+    if (ctx->bs_on_device) {   // rt_set_scene_device: the records are rebuilt where the bounding spheres are
+        if (!ctx->any_moving) return RT_OK;
+        ctx->bvh_dirty = true;
+        for (auto& d : ctx->devs) {
+            RT_CUDA(ctx, cudaSetDevice(d.dev));
+            RT_CUDA(ctx, cudaDeviceSynchronize());   // a render enqueued with sync = 0 on a caller's stream may still read the records
+            if (int rc = enqueue_records_device(ctx, d, ctx->win_lo, ctx->win_hi)) return rc;
+        }
+        for (auto& d : ctx->devs) {
+            RT_CUDA(ctx, cudaSetDevice(d.dev));
+            RT_CUDA(ctx, cudaStreamSynchronize(d.stream));
+        }
+        cudaSetDevice(ctx->devs[0].dev);
+        return RT_OK;
+    }
     bool any_moving = false;
     for (unsigned f : ctx->h_flags) any_moving |= (f & RT_SPHERE_MOVING) != 0;
     if (!any_moving) return RT_OK;
@@ -876,7 +919,29 @@ int ensure_bvh_nodes(rt_ctx* ctx, DeviceBuffers& d, size_t bytes) {
     return RT_OK;
 }
 
+// a scene of rt_set_scene_device keeps its bounding spheres on the device; the host builder reads a mirror, downloaded
+// from the first device once per scene
+int ensure_bs_mirror(rt_ctx* ctx) {
+    if (!ctx->bs_on_device || ctx->bs_mirror) return RT_OK;
+    const DeviceBuffers& d = ctx->devs[0];
+    const size_t n = (size_t)ctx->n_spheres;
+    ctx->h_bs_c0.resize(3 * n);
+    ctx->h_bs_c1.resize(3 * n);
+    ctx->h_bs_r.resize(n);
+    ctx->h_t0t1.resize(2 * n);
+    ctx->h_flags.resize(n);
+    RT_CUDA(ctx, cudaSetDevice(d.dev));
+    RT_CUDA(ctx, cudaMemcpy(ctx->h_bs_c0.data(), d.bs_in.c0, 3 * n * 8, cudaMemcpyDeviceToHost));
+    RT_CUDA(ctx, cudaMemcpy(ctx->h_bs_c1.data(), d.bs_in.c1, 3 * n * 8, cudaMemcpyDeviceToHost));
+    RT_CUDA(ctx, cudaMemcpy(ctx->h_bs_r.data(), d.bs_in.r, n * 8, cudaMemcpyDeviceToHost));
+    RT_CUDA(ctx, cudaMemcpy(ctx->h_t0t1.data(), d.bs_in.t0t1, 2 * n * 4, cudaMemcpyDeviceToHost));
+    RT_CUDA(ctx, cudaMemcpy(ctx->h_flags.data(), d.bs_in.flags, n * 4, cudaMemcpyDeviceToHost));
+    ctx->bs_mirror = true;
+    return RT_OK;
+}
+
 int bvh_build_host(rt_ctx* ctx) {
+    if (int rc = ensure_bs_mirror(ctx)) return rc;
     const int n = ctx->n_list;
     std::vector<BuildLeaf> L((size_t)n);
     for (int k = 0; k < n; ++k) {
@@ -963,17 +1028,21 @@ int bvh_enqueue_device(rt_ctx* ctx, DeviceBuffers& d) {
     }
     char* S = (char*)d.bvh_scratch;
     const cudaStream_t st = d.stream;
-    BvhLeafInput in{(const double*)(S + o_c0), (const double*)(S + o_c1), (const double*)(S + o_r), (const float*)(S + o_t),
-                    (const unsigned*)(S + o_fl)};
+    // a scene of rt_set_scene_device: the bounding spheres are already on this device
+    const BvhLeafInput in = ctx->bs_on_device ? d.bs_in
+                                              : BvhLeafInput{(const double*)(S + o_c0), (const double*)(S + o_c1), (const double*)(S + o_r),
+                                                             (const float*)(S + o_t), (const unsigned*)(S + o_fl)};
     float* boxes = (float*)(S + o_box);
     unsigned* cb = (unsigned*)(S + o_cb);
     int* depth = (int*)(S + o_depth);
     RT_CUDA(ctx, cudaEventRecord(d.ev_b0, st));
-    RT_CUDA(ctx, cudaMemcpyAsync(S + o_c0, ctx->h_bs_c0.data(), n_ * 3 * 8, cudaMemcpyHostToDevice, st));
-    RT_CUDA(ctx, cudaMemcpyAsync(S + o_c1, ctx->h_bs_c1.data(), n_ * 3 * 8, cudaMemcpyHostToDevice, st));
-    RT_CUDA(ctx, cudaMemcpyAsync(S + o_r, ctx->h_bs_r.data(), n_ * 8, cudaMemcpyHostToDevice, st));
-    RT_CUDA(ctx, cudaMemcpyAsync(S + o_t, ctx->h_t0t1.data(), n_ * 2 * 4, cudaMemcpyHostToDevice, st));
-    RT_CUDA(ctx, cudaMemcpyAsync(S + o_fl, ctx->h_flags.data(), n_ * 4, cudaMemcpyHostToDevice, st));
+    if (!ctx->bs_on_device) {
+        RT_CUDA(ctx, cudaMemcpyAsync(S + o_c0, ctx->h_bs_c0.data(), n_ * 3 * 8, cudaMemcpyHostToDevice, st));
+        RT_CUDA(ctx, cudaMemcpyAsync(S + o_c1, ctx->h_bs_c1.data(), n_ * 3 * 8, cudaMemcpyHostToDevice, st));
+        RT_CUDA(ctx, cudaMemcpyAsync(S + o_r, ctx->h_bs_r.data(), n_ * 8, cudaMemcpyHostToDevice, st));
+        RT_CUDA(ctx, cudaMemcpyAsync(S + o_t, ctx->h_t0t1.data(), n_ * 2 * 4, cudaMemcpyHostToDevice, st));
+        RT_CUDA(ctx, cudaMemcpyAsync(S + o_fl, ctx->h_flags.data(), n_ * 4, cudaMemcpyHostToDevice, st));
+    }
     RT_CUDA(ctx, cudaMemsetAsync(cb, 0xff, 3 * 4, st));   // min of the centroids: from the largest key
     RT_CUDA(ctx, cudaMemsetAsync(cb + 3, 0, 3 * 4, st));  // max: from the smallest
     const int grid = (n + 255) / 256;
@@ -1089,6 +1158,74 @@ int check_camera_times(rt_ctx* ctx) {
     return ctx->accel == RT_ACCEL_BVH ? ensure_bvh(ctx) : RT_OK;
 }
 
+// Byte offsets of the scene blob's sections: one layout for rt_set_scene_ex and rt_set_scene_device, so that both write the
+// same bytes.  Every section starts on a 256-byte boundary and takes at least 16 bytes.
+struct SceneLayout {
+    size_t cull_a, cull_tc, tc_row, c0r, c1, t0t1, orig, cull_of, flags, mat, mtype, mparam, mtex, srec, scol, tie, ttype, tparam,
+        tchild, ptype, pq, paux, pxf, xops, xp, pvec, pperm, iwh, ioff, irgb;
+    size_t bytes;
+};
+
+SceneLayout scene_layout(int n, int n_total, int n_cull, int n_direct, int tc_tiles, int nm_, int nt, int nxf, bool uses_perlin,
+                         int n_img, size_t img_bytes) {
+    SceneLayout L{};
+    size_t off = 0;
+    auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + std::max<size_t>(bytes, 16), 256); return o; };
+    L.cull_a = take((size_t)(n_cull + n_direct) * 16);
+    L.cull_tc = take((size_t)tc_tiles * tc::B_TILE_BYTES); L.tc_row = take((size_t)tc_tiles * tc::TILE_N * 4);
+    L.c0r = take((size_t)n_total * 16); L.c1 = take((size_t)n_total * 16); L.t0t1 = take((size_t)n_total * 8);
+    L.orig = take((size_t)n * 4); L.cull_of = take((size_t)n * 4); L.flags = take((size_t)n_total * 4); L.mat = take((size_t)n_total * 4);
+    L.mtype = take((size_t)nm_ * 4); L.mparam = take((size_t)nm_ * 4); L.mtex = take((size_t)nm_ * 4);
+    L.srec = take((size_t)n * 16); L.scol = take((size_t)n * 16); L.tie = take((size_t)n * 4);
+    L.ttype = take((size_t)std::max(nt, 1) * 4); L.tparam = take((size_t)std::max(nt, 1) * 48); L.tchild = take((size_t)std::max(nt, 1) * 8);
+    L.ptype = take((size_t)n_total * 4); L.pq = take((size_t)n_total * 48); L.paux = take((size_t)n_total * 8); L.pxf = take((size_t)n_total * 4);
+    L.xops = take((size_t)nxf * RT_XFORM_MAX_OPS * 4); L.xp = take((size_t)nxf * RT_XFORM_MAX_OPS * 16);
+    L.pvec = take(uses_perlin ? 256 * 16 : 0); L.pperm = take(uses_perlin ? 768 * 4 : 0);
+    L.iwh = take((size_t)n_img * 8); L.ioff = take((size_t)n_img * 8); L.irgb = take(img_bytes);
+    L.bytes = off;
+    return L;
+}
+
+// the device's scene pointers into its blob
+void set_dev_scene(DeviceBuffers& d, const SceneLayout& L, int n, int n_list, int n_cull, int tc_tiles, int generic, int n_total) {
+    char* b = (char*)d.scene_blob;
+    DevScene& sc = d.sc;
+    sc = DevScene{};
+    sc.n = n;
+    sc.n_list = n_list;
+    sc.n_cull = n_cull;
+    sc.cull_a = (const float4*)(b + L.cull_a);
+    sc.cull_tc = (const float*)(b + L.cull_tc);
+    sc.tc_row_k = (const int*)(b + L.tc_row);
+    sc.tc_tiles = tc_tiles;
+    sc.ex_c0r = (const float4*)(b + L.c0r); sc.ex_c1 = (const float4*)(b + L.c1); sc.ex_t0t1 = (const float2*)(b + L.t0t1);
+    sc.orig_id = (const int*)(b + L.orig); sc.cull_of_orig = (const int*)(b + L.cull_of);
+    sc.flags = (const unsigned*)(b + L.flags); sc.mat_id = (const int*)(b + L.mat);
+    sc.shade_rec = (const int4*)(b + L.srec); sc.shade_col = (const float4*)(b + L.scol);
+    sc.mat_type = (const int*)(b + L.mtype); sc.mat_param = (const float*)(b + L.mparam); sc.mat_tex = (const int*)(b + L.mtex);
+    sc.tex_type = (const int*)(b + L.ttype); sc.tex_params = (const float*)(b + L.tparam); sc.tex_child = (const int*)(b + L.tchild);
+    sc.generic = generic;
+    sc.n_total = n_total;
+    sc.tie_hi = (const unsigned*)(b + L.tie);
+    sc.prim_type = (const int*)(b + L.ptype); sc.prim_q = (const float4*)(b + L.pq); sc.prim_aux = (const int2*)(b + L.paux);
+    sc.prim_xform = (const int*)(b + L.pxf); sc.xform_ops = (const int*)(b + L.xops); sc.xform_p = (const float4*)(b + L.xp);
+    sc.perlin_vec = (const float4*)(b + L.pvec); sc.perlin_perm = (const int*)(b + L.pperm);
+    sc.image_wh = (const int2*)(b + L.iwh); sc.image_off = (const long long*)(b + L.ioff); sc.image_rgb = (const unsigned char*)(b + L.irgb);
+}
+
+// a device blob of at least `bytes` (and its pinned staging copy), reused by the next upload
+int ensure_scene_blob(rt_ctx* ctx, DeviceBuffers& d, size_t bytes) {
+    if (d.scene_bytes >= bytes) return RT_OK;
+    if (d.scene_blob) cudaFree(d.scene_blob);
+    if (d.scene_stage) cudaFreeHost(d.scene_stage);
+    d.scene_blob = nullptr; d.scene_stage = nullptr; d.scene_bytes = 0;
+    const size_t cap = align_up(bytes + bytes / 4, 4096);
+    RT_CUDA(ctx, cudaMalloc(&d.scene_blob, cap));
+    RT_CUDA(ctx, cudaHostAlloc(&d.scene_stage, cap, cudaHostAllocDefault));
+    d.scene_bytes = cap;
+    return RT_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1184,6 +1321,10 @@ void rt_destroy(rt_ctx* ctx) {
         if (d.bvh_nodes) cudaFree(d.bvh_nodes);
         if (d.bvh_scratch) cudaFree(d.bvh_scratch);
         if (d.h_bvh_depth) cudaFreeHost(d.h_bvh_depth);
+        if (d.bs_buf) cudaFree(d.bs_buf);
+        if (d.sb_scratch) cudaFree(d.sb_scratch);
+        if (d.h_sb) cudaFreeHost(d.h_sb);
+        if (d.ev_sb) cudaEventDestroy(d.ev_sb);
         if (d.ev_b0) cudaEventDestroy(d.ev_b0);
         if (d.ev_b1) cudaEventDestroy(d.ev_b1);
         if (d.stream) cudaStreamDestroy(d.stream);
@@ -1253,6 +1394,41 @@ static void leaf_bounds(const rt_scene_desc* s, const rt_scene_ext* x, int i, do
     }
 }
 
+// the material and texture tables of a scene (rt_set_scene_ex; x = null: rt_set_scene and rt_set_scene_device)
+static int check_tables(rt_ctx* ctx, const rt_scene_desc* s, const rt_scene_ext* x, bool* uses_perlin) {
+    const int nm_ = s->n_materials, nt = s->n_textures;
+    if (nm_ <= 0 || !s->mat_type || !s->mat_param || !s->mat_tex) return fail(ctx, RT_ERR_ARG, "material table missing");
+    if (nt < 0 || (nt > 0 && (!s->tex_type || !s->tex_params || !s->tex_children)))
+        return fail(ctx, RT_ERR_ARG, "texture table missing");
+    const int max_tex = x ? RT_TEX_IMAGE_MAP : RT_TEX_CHECKERBOARD, max_mat = x ? RT_MAT_ISOTROPIC : RT_MAT_DIFFUSE_LIGHT;
+    for (int t = 0; t < nt; ++t) {
+        int ty = s->tex_type[t];
+        if (ty < RT_TEX_CONSTANT || ty > max_tex)
+            return fail(ctx, RT_ERR_UNSUPPORTED, x ? "unknown texture type" : "texture type needs rt_set_scene_ex (texture.clj:60-138)");
+        const int n_children = ty == RT_TEX_CHECKERBOARD ? 2 : ((ty == RT_TEX_FLIP_U || ty == RT_TEX_FLIP_V) ? 1 : 0);
+        for (int c = 0; c < n_children; ++c) {
+            int ch = s->tex_children[2 * t + c];
+            if (ch < 0 || ch >= t) return fail(ctx, RT_ERR_ARG, "a texture's child must be an earlier texture id");
+        }
+        if (ty == RT_TEX_PERLIN_NOISE || ty == RT_TEX_PERLIN_TURB || ty == RT_TEX_MARBLE) *uses_perlin = true;
+        if (ty == RT_TEX_IMAGE_MAP) {
+            const int im = (int)s->tex_params[12 * t];
+            if (im < 0 || im >= x->n_images || !x->image_wh || !x->image_offset || !x->image_rgb || x->image_wh[2 * im] <= 0 ||
+                x->image_wh[2 * im + 1] <= 0)
+                return fail(ctx, RT_ERR_ARG, "image texture refers to a missing image");
+        }
+    }
+    if (*uses_perlin && (!x->perlin_vectors || !x->perlin_perm)) return fail(ctx, RT_ERR_ARG, "Perlin textures need the marshalled tables (perlin.clj:6-17)");
+    for (int m = 0; m < nm_; ++m) {
+        int ty = s->mat_type[m];
+        if (ty < RT_MAT_LAMBERTIAN || ty > max_mat)
+            return fail(ctx, RT_ERR_UNSUPPORTED, x ? "unknown material type" : "material type needs rt_set_scene_ex (shader.clj:129-143)");
+        if (ty != RT_MAT_DIELECTRIC && (s->mat_tex[m] < 0 || s->mat_tex[m] >= nt))
+            return fail(ctx, RT_ERR_ARG, "material texture id out of range");
+    }
+    return RT_OK;
+}
+
 // Upload: validate, reorder to cull order (listed leaves, then the "direct" spheres), build the FP32 cull
 // records with their conservative inflation, and copy one blob per device.
 int rt_set_scene_ex(rt_ctx* ctx, const rt_scene_desc* s, const rt_scene_ext* x) {
@@ -1264,36 +1440,8 @@ int rt_set_scene_ex(rt_ctx* ctx, const rt_scene_desc* s, const rt_scene_ext* x) 
     const int nb = x ? x->n_boundary : 0, n_total = n + nb;
     if (n <= 0 || !s->center0_r || !s->material_id) return fail(ctx, RT_ERR_ARG, "scene needs at least one primitive");
     if (nb < 0) return fail(ctx, RT_ERR_ARG, "n_boundary is negative");
-    if (nm_ <= 0 || !s->mat_type || !s->mat_param || !s->mat_tex) return fail(ctx, RT_ERR_ARG, "material table missing");
-    if (nt < 0 || (nt > 0 && (!s->tex_type || !s->tex_params || !s->tex_children)))
-        return fail(ctx, RT_ERR_ARG, "texture table missing");
-    const int max_tex = x ? RT_TEX_IMAGE_MAP : RT_TEX_CHECKERBOARD, max_mat = x ? RT_MAT_ISOTROPIC : RT_MAT_DIFFUSE_LIGHT;
     bool uses_perlin = false;
-    for (int t = 0; t < nt; ++t) {
-        int ty = s->tex_type[t];
-        if (ty < RT_TEX_CONSTANT || ty > max_tex)
-            return fail(ctx, RT_ERR_UNSUPPORTED, x ? "unknown texture type" : "texture type needs rt_set_scene_ex (texture.clj:60-138)");
-        const int n_children = ty == RT_TEX_CHECKERBOARD ? 2 : ((ty == RT_TEX_FLIP_U || ty == RT_TEX_FLIP_V) ? 1 : 0);
-        for (int c = 0; c < n_children; ++c) {
-            int ch = s->tex_children[2 * t + c];
-            if (ch < 0 || ch >= t) return fail(ctx, RT_ERR_ARG, "a texture's child must be an earlier texture id");
-        }
-        if (ty == RT_TEX_PERLIN_NOISE || ty == RT_TEX_PERLIN_TURB || ty == RT_TEX_MARBLE) uses_perlin = true;
-        if (ty == RT_TEX_IMAGE_MAP) {
-            const int im = (int)s->tex_params[12 * t];
-            if (im < 0 || im >= x->n_images || !x->image_wh || !x->image_offset || !x->image_rgb || x->image_wh[2 * im] <= 0 ||
-                x->image_wh[2 * im + 1] <= 0)
-                return fail(ctx, RT_ERR_ARG, "image texture refers to a missing image");
-        }
-    }
-    if (uses_perlin && (!x->perlin_vectors || !x->perlin_perm)) return fail(ctx, RT_ERR_ARG, "Perlin textures need the marshalled tables (perlin.clj:6-17)");
-    for (int m = 0; m < nm_; ++m) {
-        int ty = s->mat_type[m];
-        if (ty < RT_MAT_LAMBERTIAN || ty > max_mat)
-            return fail(ctx, RT_ERR_UNSUPPORTED, x ? "unknown material type" : "material type needs rt_set_scene_ex (shader.clj:129-143)");
-        if (ty != RT_MAT_DIELECTRIC && (s->mat_tex[m] < 0 || s->mat_tex[m] >= nt))
-            return fail(ctx, RT_ERR_ARG, "material texture id out of range");
-    }
+    if (int rc = check_tables(ctx, s, x, &uses_perlin)) return rc;
     const int tie_rule = x ? x->tie_rule : RT_TIE_HITLIST;
     if (tie_rule != RT_TIE_HITLIST && tie_rule != RT_TIE_BVH) return fail(ctx, RT_ERR_ARG, "unknown tie rule");
     int generic = uses_perlin ? 1 : 0;
@@ -1469,13 +1617,9 @@ int rt_set_scene_ex(rt_ctx* ctx, const rt_scene_desc* s, const rt_scene_ext* x) 
     ctx->n_total = n_total;
     ctx->generic = generic;
 
-    // blob layout
-    size_t off = 0;
-    auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + std::max<size_t>(bytes, 16), 256); return o; };
-    size_t o_cull_a = take((size_t)(n_cull + n_direct) * 16);
     const int tc_tiles = (n_list + tc::TILE_N - 1) / tc::TILE_N;   // (over MAX_TILES: several wf_cull_tc launches per iteration)
     ctx->tc_tiles = tc_tiles;
-    size_t o_cull_tc = take((size_t)tc_tiles * tc::B_TILE_BYTES), o_tc_row = take((size_t)tc_tiles * tc::TILE_N * 4);
+    ctx->bs_on_device = ctx->bs_mirror = false;
     {   // rows: the listed leaves dealt out over the 32-row words largest first (a leaf's share of the candidates grows with its
         // radius), so that every epilogue warp's columns see the same mix; the padding rows are spread the same way
         ctx->tc_row_k.assign((size_t)tc_tiles * tc::TILE_N, -1);
@@ -1488,20 +1632,17 @@ int rt_set_scene_ex(rt_ctx* ctx, const rt_scene_desc* s, const rt_scene_ext* x) 
             for (int i = 0; i < n_list; ++i) ctx->tc_row_k[(size_t)(i % words) * 32 + (size_t)(i / words)] = order[(size_t)i];
         }
     }
-    size_t o_c0r = take((size_t)n_total * 16), o_c1 = take((size_t)n_total * 16), o_t0t1 = take((size_t)n_total * 8);
-    size_t o_orig = take((size_t)n * 4), o_cull_of = take((size_t)n * 4), o_flags = take((size_t)n_total * 4), o_mat = take((size_t)n_total * 4);
-    size_t o_mtype = take((size_t)nm_ * 4), o_mparam = take((size_t)nm_ * 4), o_mtex = take((size_t)nm_ * 4);
-    size_t o_srec = take((size_t)n * 16), o_scol = take((size_t)n * 16), o_tie = take((size_t)n * 4);
-    size_t o_ttype = take((size_t)std::max(nt, 1) * 4), o_tparam = take((size_t)std::max(nt, 1) * 48), o_tchild = take((size_t)std::max(nt, 1) * 8);
     const int nxf = x ? std::max(0, x->n_xforms) : 0;
-    size_t o_ptype = take((size_t)n_total * 4), o_pq = take((size_t)n_total * 48), o_paux = take((size_t)n_total * 8), o_pxf = take((size_t)n_total * 4);
-    size_t o_xops = take((size_t)nxf * RT_XFORM_MAX_OPS * 4), o_xp = take((size_t)nxf * RT_XFORM_MAX_OPS * 16);
-    size_t o_pvec = take(uses_perlin ? 256 * 16 : 0), o_pperm = take(uses_perlin ? 768 * 4 : 0);
     const int n_img = x ? std::max(0, x->n_images) : 0;
     size_t img_bytes = 0;
     for (int i = 0; i < n_img; ++i) img_bytes = std::max(img_bytes, (size_t)x->image_offset[i] + (size_t)x->image_wh[2 * i] * x->image_wh[2 * i + 1] * 3);
-    size_t o_iwh = take((size_t)n_img * 8), o_ioff = take((size_t)n_img * 8), o_irgb = take(img_bytes);
-    std::vector<unsigned char> blob(off, 0);
+    const SceneLayout L = scene_layout(n, n_total, n_cull, n_direct, tc_tiles, nm_, nt, nxf, uses_perlin, n_img, img_bytes);
+    const size_t o_cull_a = L.cull_a, o_cull_tc = L.cull_tc, o_tc_row = L.tc_row, o_c0r = L.c0r, o_c1 = L.c1, o_t0t1 = L.t0t1;
+    const size_t o_orig = L.orig, o_cull_of = L.cull_of, o_flags = L.flags, o_mat = L.mat, o_mtype = L.mtype, o_mparam = L.mparam;
+    const size_t o_mtex = L.mtex, o_srec = L.srec, o_scol = L.scol, o_tie = L.tie, o_ttype = L.ttype, o_tparam = L.tparam;
+    const size_t o_tchild = L.tchild, o_ptype = L.ptype, o_pq = L.pq, o_paux = L.paux, o_pxf = L.pxf, o_xops = L.xops, o_xp = L.xp;
+    const size_t o_pvec = L.pvec, o_pperm = L.pperm, o_iwh = L.iwh, o_ioff = L.ioff, o_irgb = L.irgb;
+    std::vector<unsigned char> blob(L.bytes, 0);
     build_cull_records(ctx, win_lo, win_hi, (float*)(blob.data() + o_cull_a), tc_tiles ? (float*)(blob.data() + o_cull_tc) : nullptr);
     if (tc_tiles) memcpy(blob.data() + o_tc_row, ctx->tc_row_k.data(), ctx->tc_row_k.size() * 4);
     memcpy(blob.data() + o_c0r, ctx->h_c0r.data(), (size_t)n_total * 16);
@@ -1573,41 +1714,12 @@ int rt_set_scene_ex(rt_ctx* ctx, const rt_scene_desc* s, const rt_scene_ext* x) 
     for (auto& d : ctx->devs) {
         RT_CUDA(ctx, cudaSetDevice(d.dev));
         RT_CUDA(ctx, cudaDeviceSynchronize());   // renders enqueued with sync = 0 on a caller's stream may still read the old scene
-        if (d.scene_bytes < blob.size()) {       // the blob (and its pinned staging copy) is reused by the next upload
-            if (d.scene_blob) cudaFree(d.scene_blob);
-            if (d.scene_stage) cudaFreeHost(d.scene_stage);
-            d.scene_blob = nullptr; d.scene_stage = nullptr; d.scene_bytes = 0;
-            const size_t cap = align_up(blob.size() + blob.size() / 4, 4096);
-            RT_CUDA(ctx, cudaMalloc(&d.scene_blob, cap));
-            RT_CUDA(ctx, cudaHostAlloc(&d.scene_stage, cap, cudaHostAllocDefault));
-            d.scene_bytes = cap;
-        }
+        if (int rc = ensure_scene_blob(ctx, d, blob.size())) return rc;
         memcpy(d.scene_stage, blob.data(), blob.size());
         RT_CUDA(ctx, cudaMemcpyAsync(d.scene_blob, d.scene_stage, blob.size(), cudaMemcpyHostToDevice, d.stream));
         RT_CUDA(ctx, cudaStreamSynchronize(d.stream));
-        char* b = (char*)d.scene_blob;
-        DevScene& sc = d.sc;
-        sc = DevScene{};
-        sc.n = n;
-        sc.n_list = n_list;
-        sc.n_cull = n_cull;
-        sc.cull_a = (const float4*)(b + o_cull_a);
-        sc.cull_tc = (const float*)(b + o_cull_tc);
-        sc.tc_row_k = (const int*)(b + o_tc_row);
-        sc.tc_tiles = tc_tiles;
-        sc.ex_c0r = (const float4*)(b + o_c0r); sc.ex_c1 = (const float4*)(b + o_c1); sc.ex_t0t1 = (const float2*)(b + o_t0t1);
-        sc.orig_id = (const int*)(b + o_orig); sc.cull_of_orig = (const int*)(b + o_cull_of);
-        sc.flags = (const unsigned*)(b + o_flags); sc.mat_id = (const int*)(b + o_mat);
-        sc.shade_rec = (const int4*)(b + o_srec); sc.shade_col = (const float4*)(b + o_scol);
-        sc.mat_type = (const int*)(b + o_mtype); sc.mat_param = (const float*)(b + o_mparam); sc.mat_tex = (const int*)(b + o_mtex);
-        sc.tex_type = (const int*)(b + o_ttype); sc.tex_params = (const float*)(b + o_tparam); sc.tex_child = (const int*)(b + o_tchild);
-        sc.generic = generic;
-        sc.n_total = n_total;
-        sc.tie_hi = (const unsigned*)(b + o_tie);
-        sc.prim_type = (const int*)(b + o_ptype); sc.prim_q = (const float4*)(b + o_pq); sc.prim_aux = (const int2*)(b + o_paux);
-        sc.prim_xform = (const int*)(b + o_pxf); sc.xform_ops = (const int*)(b + o_xops); sc.xform_p = (const float4*)(b + o_xp);
-        sc.perlin_vec = (const float4*)(b + o_pvec); sc.perlin_perm = (const int*)(b + o_pperm);
-        sc.image_wh = (const int2*)(b + o_iwh); sc.image_off = (const long long*)(b + o_ioff); sc.image_rgb = (const unsigned char*)(b + o_irgb);
+        d.scene_used = blob.size();
+        set_dev_scene(d, L, n, n_list, n_cull, tc_tiles, generic, n_total);
     }
     cudaSetDevice(ctx->devs[0].dev);
     // resident up to kTileCap records; beyond that the list is streamed through a smaller tile (tile_records,
@@ -1623,6 +1735,206 @@ int rt_set_scene_ex(rt_ctx* ctx, const rt_scene_desc* s, const rt_scene_ext* x) 
 }
 
 int rt_set_scene(rt_ctx* ctx, const rt_scene_desc* s) { return rt_set_scene_ex(ctx, s, nullptr); }
+
+// rt_set_scene with the per-primitive arrays in device memory: rt_set_scene_ex's steps for a sphere scene, run on the first
+// device (rt_scene_build.cuh); the blob and the bounding spheres then go to every other device by peer copies.  Nothing but
+// the tables and a small result crosses the host link.
+int rt_set_scene_device(rt_ctx* ctx, const rt_scene_desc* s, void* stream) {
+    if (!ctx) return RT_ERR_ARG;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    if (!s) return fail(ctx, RT_ERR_ARG, "scene is null");
+    const int n = s->n_spheres, nm_ = s->n_materials, nt = s->n_textures;
+    if (n <= 0 || !s->center0_r || !s->material_id) return fail(ctx, RT_ERR_ARG, "scene needs at least one primitive");
+    bool uses_perlin = false;
+    if (int rc = check_tables(ctx, s, nullptr, &uses_perlin)) return rc;
+    DeviceBuffers& d0 = ctx->devs[0];
+    RT_CUDA(ctx, cudaSetDevice(d0.dev));
+    for (const void* p : {(const void*)s->center0_r, (const void*)s->center1, (const void*)s->t0t1, (const void*)s->sphere_flags,
+                          (const void*)s->material_id}) {
+        if (!p) continue;
+        cudaPointerAttributes a{};
+        const cudaError_t e = cudaPointerGetAttributes(&a, p);
+        if (e != cudaSuccess) cudaGetLastError();   // not a pointer the runtime knows: clear the error, reject below
+        if (e != cudaSuccess || (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) || a.device != d0.dev)
+            return fail(ctx, RT_ERR_ARG, "rt_set_scene_device: a per-primitive array is not device memory on the context's first device");
+    }
+
+    // scratch of the first device: result | radii | sorted radii | partial sums | candidates | candidate count | cull order |
+    // radius keys and leaf values of the feature-row sort (in, out) | cub storage
+    const size_t n_ = (size_t)n;
+    const bool want_direct = n > 16 && ctx->opt.direct_spheres;
+    const cudaStream_t st = d0.stream;
+    size_t sort_cap = 0;   // both sorts: (u64 key, int) pairs; radii are non-negative, so their bits sort as their values
+    RT_CUDA(ctx, cub::DeviceRadixSort::SortPairs(nullptr, sort_cap, (const unsigned long long*)nullptr, (unsigned long long*)nullptr,
+                                                 (const int*)nullptr, (int*)nullptr, n, 0, 64, st));
+    size_t off = 0;
+    auto take = [&](size_t bytes) { const size_t o = off; off = align_up(off + bytes, 256); return o; };
+    const size_t o_res = take(sizeof(SbResult)), o_rad = take(n_ * 8), o_sorted = take(n_ * 8), o_part = take((size_t)kSbPartials * 4 * 8);
+    const size_t o_cand = take(n_ * 4), o_ncand = take(4), o_perm = take(n_ * 4), o_key = take(n_ * 8), o_key2 = take(n_ * 8);
+    const size_t o_val = take(n_ * 4), o_val2 = take(n_ * 4), o_sort = take(sort_cap);
+    if (d0.sb_scratch_bytes < off) {
+        if (d0.sb_scratch) cudaFree(d0.sb_scratch);
+        d0.sb_scratch = nullptr;
+        d0.sb_scratch_bytes = 0;
+        RT_CUDA(ctx, cudaMalloc(&d0.sb_scratch, off));
+        d0.sb_scratch_bytes = off;
+    }
+    if (!d0.h_sb) {
+        RT_CUDA(ctx, cudaHostAlloc((void**)&d0.h_sb, sizeof(SbResult), cudaHostAllocDefault));
+        RT_CUDA(ctx, cudaEventCreateWithFlags(&d0.ev_sb, cudaEventDisableTiming));
+    }
+    char* W = (char*)d0.sb_scratch;
+    SbResult* res = (SbResult*)(W + o_res);
+    double* radii = (double*)(W + o_rad);
+    double* sorted = (double*)(W + o_sorted);
+    int* perm = (int*)(W + o_perm);
+    const SbInput in{s->center0_r, s->center1, s->t0t1, s->sphere_flags, s->material_id, n, nm_};
+    const int grid = (n + kSbBlock - 1) / kSbBlock;
+
+    // 1. validation and the movers' window, 2. the direct spheres; one small read-back
+    RT_CUDA(ctx, cudaEventRecord(d0.ev_sb, (cudaStream_t)stream));   // the caller's writes to the arrays come first
+    RT_CUDA(ctx, cudaStreamWaitEvent(st, d0.ev_sb, 0));
+    *d0.h_sb = SbResult{~0ull, 0xffffffffu, 0u, 0, {}, {}};
+    RT_CUDA(ctx, cudaMemcpyAsync(res, d0.h_sb, sizeof(SbResult), cudaMemcpyHostToDevice, st));
+    sb_validate<<<grid, kSbBlock, 0, st>>>(in, res, want_direct ? radii : nullptr);
+    if (want_direct) {
+        size_t sort_bytes = sort_cap;   // (the values are scratch: only the sorted radii are used)
+        RT_CUDA(ctx, cub::DeviceRadixSort::SortPairs(W + o_sort, sort_bytes, (const unsigned long long*)radii, (unsigned long long*)sorted,
+                                                     (const int*)(W + o_val), (int*)(W + o_val2), n, 0, 64, st));
+        sb_small_partials<<<kSbPartials, kSbBlock, 0, st>>>(in, radii, sorted, (double*)(W + o_part));
+        sb_centroid<<<1, kSbPartials, 0, st>>>((const double*)(W + o_part), res);
+        RT_CUDA(ctx, cudaMemsetAsync(W + o_ncand, 0, 4, st));
+        sb_candidates<<<grid, kSbBlock, 0, st>>>(in, radii, sorted, res, (int*)(W + o_cand), (unsigned*)(W + o_ncand));
+        sb_direct_choose<<<1, 32, 0, st>>>(in, radii, (const int*)(W + o_cand), (const unsigned*)(W + o_ncand), res);
+    }
+    RT_CUDA(ctx, cudaGetLastError());
+    RT_CUDA(ctx, cudaMemcpyAsync(d0.h_sb, res, sizeof(SbResult), cudaMemcpyDeviceToHost, st));
+    RT_CUDA(ctx, cudaStreamSynchronize(st));
+    const SbResult R = *d0.h_sb;
+    if (R.err != ~0ull) {   // the first failing primitive, its first failing check: the host loop's error
+        const int check = (int)(R.err & 3ull);
+        if (check == 0) return fail(ctx, RT_ERR_UNSUPPORTED, "unknown sphere flag");
+        return fail(ctx, RT_ERR_ARG, check == 1 ? "material id out of range" : "moving sphere with t1 == t0");
+    }
+    auto unordered = [](unsigned u) {
+        u = (u & 0x80000000u) ? (u & 0x7fffffffu) : ~u;
+        float f;
+        memcpy(&f, &u, 4);
+        return (double)f;
+    };
+    const bool any_moving = R.win_hi >= R.win_lo;
+    double win_lo = any_moving ? unordered(R.win_lo) : 0.0, win_hi = any_moving ? unordered(R.win_hi) : 0.0;
+    if (ctx->has_cam) {   // cover the shutter interval already set
+        double lo = ctx->cam.type == CAM_THIN_LENS ? std::min(ctx->cam.t0, ctx->cam.t1) : 0.0;
+        double hi = ctx->cam.type == CAM_THIN_LENS ? std::max(ctx->cam.t0, ctx->cam.t1) : 0.0;
+        win_lo = std::min(win_lo, lo);
+        win_hi = std::max(win_hi, hi);
+    }
+    const int n_direct = want_direct ? R.n_direct : 0;
+    const int n_list = n - n_direct;
+    const int n_cull = (int)align_up((size_t)n_list, CULL_PAD);
+    const int tc_tiles = (n_list + tc::TILE_N - 1) / tc::TILE_N, rows = tc_tiles * tc::TILE_N;
+    const SceneLayout L = scene_layout(n, n, n_cull, n_direct, tc_tiles, nm_, nt, 0, false, 0, 0);
+    const size_t bs_bytes = n_ * 7 * 8;   // c0 [3n], c1 [3n], r [n]
+
+    for (auto& d : ctx->devs) {
+        RT_CUDA(ctx, cudaSetDevice(d.dev));
+        RT_CUDA(ctx, cudaDeviceSynchronize());   // renders enqueued with sync = 0 on a caller's stream may still read the old scene
+        if (int rc = ensure_scene_blob(ctx, d, L.bytes)) return rc;
+        if (d.bs_bytes < bs_bytes) {
+            if (d.bs_buf) cudaFree(d.bs_buf);
+            d.bs_buf = nullptr;
+            d.bs_bytes = 0;
+            RT_CUDA(ctx, cudaMalloc(&d.bs_buf, bs_bytes));
+            d.bs_bytes = bs_bytes;
+        }
+    }
+    RT_CUDA(ctx, cudaSetDevice(d0.dev));
+    ctx->n_list = n_list;
+    ctx->n_cull = n_cull;
+    ctx->n_spheres = n;
+    ctx->n_total = n;
+    ctx->generic = 0;
+    ctx->tc_tiles = tc_tiles;
+    ctx->tc_row_k.clear();
+    ctx->tc_scratch_rows.clear();
+    ctx->bs_on_device = true;
+    ctx->bs_mirror = false;
+    ctx->any_moving = any_moving;
+    for (auto& d : ctx->devs) {
+        set_dev_scene(d, L, n, n_list, n_cull, tc_tiles, 0, n);
+        double* bs = (double*)d.bs_buf;
+        d.bs_in = BvhLeafInput{bs, bs + 3 * n_, bs + 6 * n_, (const float*)d.sc.ex_t0t1, d.sc.flags};
+        d.scene_used = L.bytes;
+    }
+
+    // 3. the blob, zeroed (the host's blob is a zero-filled vector), with the tables staged through pinned memory
+    char* B = (char*)d0.scene_blob;
+    char* S = (char*)d0.scene_stage;
+    RT_CUDA(ctx, cudaMemsetAsync(B, 0, L.bytes, st));
+    auto table = [&](size_t o, const void* src, size_t bytes) -> cudaError_t {
+        memcpy(S + o, src, bytes);
+        return cudaMemcpyAsync(B + o, S + o, bytes, cudaMemcpyHostToDevice, st);
+    };
+    RT_CUDA(ctx, table(L.mtype, s->mat_type, (size_t)nm_ * 4));
+    RT_CUDA(ctx, table(L.mparam, s->mat_param, (size_t)nm_ * 4));
+    RT_CUDA(ctx, table(L.mtex, s->mat_tex, (size_t)nm_ * 4));
+    if (nt > 0) {
+        RT_CUDA(ctx, table(L.ttype, s->tex_type, (size_t)nt * 4));
+        RT_CUDA(ctx, table(L.tparam, s->tex_params, (size_t)nt * 48));
+        RT_CUDA(ctx, table(L.tchild, s->tex_children, (size_t)nt * 8));
+    }
+    if (n_direct) sb_perm<<<grid, kSbBlock, 0, st>>>(n, res, perm);
+    unsigned long long* key = (unsigned long long*)(W + o_key);
+    int* val = (int*)(W + o_val);
+    const SbBlob blob{(float*)(B + L.c0r), (float*)(B + L.c1), (float*)(B + L.t0t1), (unsigned*)(B + L.flags), (int*)(B + L.mat),
+                      (int*)(B + L.orig), (int*)(B + L.cull_of), (int*)(B + L.srec), (float*)(B + L.scol), (unsigned*)(B + L.tie),
+                      (const int*)(B + L.mtype), (const float*)(B + L.mparam), (const int*)(B + L.mtex), (const int*)(B + L.ttype),
+                      (const float*)(B + L.tparam), nt, (double*)d0.bs_in.c0, (double*)d0.bs_in.c1, (double*)d0.bs_in.r, key, val, n_list};
+    sb_gather<<<grid, kSbBlock, 0, st>>>(in, n_direct ? perm : nullptr, blob);
+    // 4. the feature rows: listed leaves by bounding radius, descending, stable; dealt over the 32-row words
+    size_t sort_bytes = 0;
+    RT_CUDA(ctx, cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, (const unsigned long long*)nullptr, (unsigned long long*)nullptr,
+                                                 (const int*)nullptr, (int*)nullptr, n_list, 0, 64, st));
+    if (sort_bytes > sort_cap) return fail(ctx, RT_ERR_STATE, "rt_set_scene_device: sort storage underestimated");
+    RT_CUDA(ctx, cub::DeviceRadixSort::SortPairs(W + o_sort, sort_bytes, key, (unsigned long long*)(W + o_key2), val, (int*)(W + o_val2),
+                                                 n_list, 0, 64, st));
+    sb_deal<<<(rows + kSbBlock - 1) / kSbBlock, kSbBlock, 0, st>>>((const int*)(W + o_val2), n_list, rows, (int*)(B + L.tc_row));
+    RT_CUDA(ctx, cudaGetLastError());
+    // 5. the cull records, the padding records and the rows' slots
+    if (int rc = enqueue_records_device(ctx, d0, win_lo, win_hi)) return rc;
+    // every other device: the same bytes
+    for (size_t q = 1; q < ctx->devs.size(); ++q) {
+        DeviceBuffers& d = ctx->devs[q];
+        RT_CUDA(ctx, cudaMemcpyPeerAsync(d.scene_blob, d.dev, d0.scene_blob, d0.dev, L.bytes, st));
+        RT_CUDA(ctx, cudaMemcpyPeerAsync(d.bs_buf, d.dev, d0.bs_buf, d0.dev, bs_bytes, st));
+    }
+    RT_CUDA(ctx, cudaStreamSynchronize(st));
+    const int tile_records = std::max(CHUNK, std::min(kTileCap, ctx->opt.tile_records / CHUNK * CHUNK));
+    ctx->preloaded = n_cull <= kTileCap ? 1 : 0;
+    ctx->cull_cap = ctx->preloaded ? std::max(n_cull, CULL_PAD) : tile_records;
+    ctx->win_lo = win_lo;
+    ctx->win_hi = win_hi;
+    ctx->has_scene = true;
+    ctx->bvh_dirty = true;
+    return RT_OK;
+}
+
+int rt_get_scene_blob(rt_ctx* ctx, int device_index, void* out, size_t cap, size_t* bytes) {
+    if (!ctx) return RT_ERR_ARG;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    if (int rc = check_ready(ctx)) return rc;
+    if (device_index < 0 || device_index >= (int)ctx->devs.size()) return fail(ctx, RT_ERR_ARG, "device_index out of range");
+    const DeviceBuffers& d = ctx->devs[(size_t)device_index];
+    if (bytes) *bytes = d.scene_used;
+    if (out) {
+        if (cap < d.scene_used) return fail(ctx, RT_ERR_ARG, "cap is below the blob's size (*bytes)");
+        RT_CUDA(ctx, cudaSetDevice(d.dev));
+        RT_CUDA(ctx, cudaMemcpy(out, d.scene_blob, d.scene_used, cudaMemcpyDeviceToHost));
+        cudaSetDevice(ctx->devs[0].dev);
+    }
+    return RT_OK;
+}
 
 int rt_set_accel(rt_ctx* ctx, int accel) {
     if (!ctx) return RT_ERR_ARG;

@@ -125,18 +125,36 @@ __device__ __forceinline__ void split2(float x, float& hi, float& lo) {
 //   0 g0.hi|1     1 g0.lo|1     2 1|W.hi      3 1|W.lo      4 gx.hi|cx.hi   5 gx.hi|cx.lo   6 gx.lo|cx.hi   7 1|W.lo2
 //   8 gy.hi|cy.hi 9 gy.hi|cy.lo 10 gy.lo|cy.hi 11 qyz.hi|cyz.lo  12 gz.hi|cz.hi 13 gz.hi|cz.lo 14 gz.lo|cz.hi 15 qyz.lo|cyz.hi
 //   16..18 qxx|cxx   19..21 qyy|cyy   22..24 qzz|czz   25..27 qxy|cxy   28..30 qxz|cxz  (hi|hi, hi|lo, lo|hi)   31 qyz.hi|cyz.hi
-// Host side: one sphere's 32 slots (build_cull_records).  c = centre AS STORED in the FP32 record, W in double.
-inline void sphere_slots(const double c[3], double W, float out[KTOT]) {
-    auto sp2 = [](double x, float& hi, float& lo) { hi = tf32_rn((float)x); lo = tf32_rn((float)(x - (double)hi)); };
-    float wh = tf32_rn((float)W), wl = tf32_rn((float)(W - (double)wh)), wl2 = tf32_rn((float)(W - (double)wh - (double)wl));
+// FP64 product / difference rounded as written on both sides: the device must not contract them into an FMA
+__host__ __device__ inline double dmul_rn(double a, double b) {
+#ifdef __CUDA_ARCH__
+    return __dmul_rn(a, b);
+#else
+    return a * b;
+#endif
+}
+__host__ __device__ inline double dsub_rn(double a, double b) {
+#ifdef __CUDA_ARCH__
+    return __dsub_rn(a, b);
+#else
+    return a - b;
+#endif
+}
+
+// One sphere's 32 slots (build_cull_records on the host, sb_tc_rows on the device: the same bits).  c = centre AS STORED in
+// the FP32 record, W in double.
+__host__ __device__ inline void sphere_slots(const double c[3], double W, float out[KTOT]) {
+    auto sp2 = [](double x, float& hi, float& lo) { hi = tf32_rn((float)x); lo = tf32_rn((float)dsub_rn(x, (double)hi)); };
+    float wh = tf32_rn((float)W), wl = tf32_rn((float)dsub_rn(W, (double)wh)), wl2 = tf32_rn((float)dsub_rn(dsub_rn(W, (double)wh), (double)wl));
     float ch[3], cl[3], dh[3], dl[3], eh[3], el[3];   // c_i, c_i^2, cross terms (xy, xz, yz)
-    for (int i = 0; i < 3; ++i) { sp2(c[i], ch[i], cl[i]); sp2(c[i] * c[i], dh[i], dl[i]); }
-    sp2(2.0 * c[0] * c[1], eh[0], el[0]); sp2(2.0 * c[0] * c[2], eh[1], el[1]); sp2(2.0 * c[1] * c[2], eh[2], el[2]);
+    for (int i = 0; i < 3; ++i) { sp2(c[i], ch[i], cl[i]); sp2(dmul_rn(c[i], c[i]), dh[i], dl[i]); }
+    sp2(dmul_rn(dmul_rn(2.0, c[0]), c[1]), eh[0], el[0]); sp2(dmul_rn(dmul_rn(2.0, c[0]), c[2]), eh[1], el[1]);
+    sp2(dmul_rn(dmul_rn(2.0, c[1]), c[2]), eh[2], el[2]);
     const float s[KTOT] = {1.f, 1.f, wh, wl, ch[0], cl[0], ch[0], wl2, ch[1], cl[1], ch[1], el[2], ch[2], cl[2], ch[2], eh[2],
                            dh[0], dl[0], dh[0], dh[1], dl[1], dh[1], dh[2], dl[2], dh[2], eh[0], el[0], eh[0], eh[1], el[1], eh[1], eh[2]};
     for (int k = 0; k < KTOT; ++k) out[k] = s[k];
 }
-inline void padding_slots(float out[KTOT]) {
+__host__ __device__ inline void padding_slots(float out[KTOT]) {
     for (int k = 0; k < KTOT; ++k) out[k] = 0.f;
     out[0] = 1.f;                      // against g0.hi: a DEAD ray stays dead (0 x 0 would be +0 = "candidate")
     out[2] = DEAD;                     // W.hi against the ray's 1

@@ -111,6 +111,22 @@ class FlatScene:
     def nbytes(self):
         return int(sum(getattr(self, k).nbytes for k in self.__dataclass_fields__ if isinstance(getattr(self, k), np.ndarray)))
 
+    def sphere_tensors(self, device):
+        """The five per-primitive arrays as torch CUDA tensors on `device`, in the dtypes and shapes
+        ``Renderer.set_scene_device`` takes (sphere_flags as int32: the same bits)."""
+        import torch
+        c = np.ascontiguousarray
+        return dict(center0_r=torch.from_numpy(c(self.center0_r, np.float32)).to(device),
+                    center1=torch.from_numpy(c(self.center1, np.float32)).to(device),
+                    t0t1=torch.from_numpy(c(self.t0t1, np.float32)).to(device),
+                    sphere_flags=torch.from_numpy(c(self.sphere_flags, np.uint32).view(np.int32)).to(device),
+                    material_id=torch.from_numpy(c(self.material_id, np.int32)).to(device))
+
+    def tables(self):
+        """The material and texture tables (host arrays), as ``Renderer.set_scene_device`` takes them."""
+        return dict(mat_type=self.mat_type, mat_param=self.mat_param, mat_tex=self.mat_tex, tex_type=self.tex_type,
+                    tex_params=self.tex_params, tex_children=self.tex_children)
+
 
 _LEAF_TYPES = (hit.Sphere, hit.MovingSphere, hit.RectXY, hit.RectXZ, hit.RectYZ, hit.Triangle, hit.ConstantMedium)
 
@@ -380,7 +396,7 @@ ABI_SYMBOLS = [
     "rt_render_accumulate_device", "rt_resolve_device", "rt_trace_primary", "rt_generate_rays", "rt_shade_batch",
     "rt_measure_fp32_peak", "rt_get_counters", "rt_reset_counters", "rt_set_profile", "rt_device_info", "rt_cull_check",
     "rt_set_scene_ex", "rt_trace_paths", "rt_set_accel", "rt_set_option", "rt_sample_device", "rt_host_alloc", "rt_host_free",
-    "rt_get_bvh",
+    "rt_get_bvh", "rt_set_scene_device", "rt_get_scene_blob",
 ]
 
 _lib = None
@@ -427,6 +443,8 @@ def load_library():
     L.rt_host_alloc.argtypes = [C.c_void_p, C.c_size_t, C.POINTER(C.c_void_p)]
     L.rt_host_free.argtypes = [C.c_void_p, C.c_void_p]
     L.rt_get_bvh.argtypes = [C.c_void_p, C.c_int, _f32p, C.c_int64, C.POINTER(C.c_int64)]
+    L.rt_set_scene_device.argtypes = [C.c_void_p, C.POINTER(_SceneDesc), C.c_void_p]
+    L.rt_get_scene_blob.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)]
     _lib = L
     return L
 
@@ -442,6 +460,7 @@ class Renderer:
         self.L = load_library()
         self.h = C.c_void_p()
         ids = np.asarray(device_ids if device_ids is not None else [0], np.int32)
+        self.device_ids = [int(i) for i in ids]
         rc = self.L.rt_create(C.byref(self.h), _p(ids, _i32p), C.c_int(len(ids)))
         if rc != 0:
             msg = self.L.rt_last_error(None)
@@ -534,6 +553,60 @@ class Renderer:
             self._check(self.L.rt_set_scene(self.h, C.byref(d)), "rt_set_scene")
         else:
             self._check(self.L.rt_set_scene_ex(self.h, C.byref(d), C.byref(x)), "rt_set_scene_ex")
+
+    def set_scene_device(self, center0_r, material_id, mat_type, mat_param, mat_tex, tex_type, tex_params, tex_children,
+                         center1=None, t0t1=None, sphere_flags=None, stream=None):
+        """rt_set_scene_device: the per-primitive arrays are torch CUDA tensors on the context's first device (center0_r /
+        center1 [n,4] float32, t0t1 [n,2] float32, sphere_flags [n] int32 or uint32, material_id [n] int32, contiguous); the
+        tables are host arrays.  The GPU builds the scene blob rt_set_scene would upload for the same values.  The library
+        reads the tensors after the work already queued on `stream` (default: torch's current stream) and returns once the
+        scene is built, so they may be changed right after.  Sphere scenes of rt_set_scene only (no rt_scene_ext): exact ties
+        go to the first sphere in caller order (RT_TIE_HITLIST), also for arrays marshalled from a bvh-node world, whose
+        FlatScene carries RT_TIE_BVH for rt_set_scene_ex."""
+        import torch
+        dev = torch.device("cuda", self.device_ids[0])
+        n = center0_r.shape[0] if isinstance(center0_r, torch.Tensor) and center0_r.dim() == 2 else None
+
+        def check(name, t, dtypes, cols):
+            if t is None:
+                return None
+            if not isinstance(t, torch.Tensor) or t.device != dev:
+                raise ValueError(f"{name} must be a torch tensor on {dev}")
+            if t.dtype not in dtypes:
+                raise ValueError(f"{name} must be {' or '.join(str(d) for d in dtypes)}, not {t.dtype}")
+            shape = (n,) if cols is None else (n, cols)
+            if tuple(t.shape) != shape:
+                raise ValueError(f"{name} must have shape {shape}, not {tuple(t.shape)}")
+            if not t.is_contiguous():
+                raise ValueError(f"{name} must be contiguous")
+            return C.c_void_p(t.data_ptr())
+
+        if n is None or n == 0:
+            raise ValueError("center0_r must be a [n,4] tensor with n >= 1")
+        ptr = dict(c0=check("center0_r", center0_r, (torch.float32,), 4), c1=check("center1", center1, (torch.float32,), 4),
+                   tt=check("t0t1", t0t1, (torch.float32,), 2),
+                   fl=check("sphere_flags", sphere_flags, (torch.int32, getattr(torch, "uint32", torch.int32)), None),
+                   mi=check("material_id", material_id, (torch.int32,), None))
+        c = np.ascontiguousarray
+        k = dict(mt=c(mat_type, np.int32), mp=c(mat_param, np.float32), mx=c(mat_tex, np.int32), tt2=c(tex_type, np.int32),
+                 tp=c(tex_params, np.float32), tc=c(tex_children, np.int32))
+        cast = lambda p, ty: C.cast(p, ty) if p is not None else None
+        d = _SceneDesc(n, cast(ptr["c0"], _f32p), cast(ptr["c1"], _f32p), cast(ptr["tt"], _f32p), cast(ptr["fl"], _u32p),
+                       cast(ptr["mi"], _i32p), len(k["mt"]), _p(k["mt"], _i32p), _p(k["mp"], _f32p), _p(k["mx"], _i32p),
+                       len(k["tt2"]), _p(k["tt2"], _i32p), _p(k["tp"], _f32p), _p(k["tc"], _i32p))
+        if stream is None:
+            stream = torch.cuda.current_stream(dev).cuda_stream
+        self.flat = None
+        self._check(self.L.rt_set_scene_device(self.h, C.byref(d), C.c_void_p(int(stream) or None)), "rt_set_scene_device")
+
+    def scene_blob(self, device_index=0):
+        """rt_get_scene_blob: the scene blob one device of the context holds, as uint8 (diagnostic)."""
+        nbytes = C.c_size_t(0)
+        self._check(self.L.rt_get_scene_blob(self.h, int(device_index), None, 0, C.byref(nbytes)), "rt_get_scene_blob")
+        out = np.zeros(nbytes.value, np.uint8)
+        self._check(self.L.rt_get_scene_blob(self.h, int(device_index), out.ctypes.data_as(C.c_void_p), nbytes, C.byref(nbytes)),
+                    "rt_get_scene_blob")
+        return out
 
     def set_accel(self, accel):
         """RT_ACCEL_BRUTE_FORCE (the roofline path) or RT_ACCEL_BVH (flattened GPU BVH, hitable.clj:97-123's role)."""
