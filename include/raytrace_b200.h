@@ -198,6 +198,9 @@ enum {
                                 from the culled tests; RT_CTR_SPHERE_TESTS = rays * n still counts every pair once)   */
     RT_CTR_BVH_NODE_TESTS,   /* RT_ACCEL_BVH: box tests (the reference's `aabb.intersection.total`, metrics.clj:9)     */
     RT_CTR_REDUCE_NS,        /* multi-device rt_render: device time of the cross-device reduce, ns                     */
+    RT_CTR_COMMON_ORIGIN_RAYS, /* wavefront camera rays whose cameras all share one origin, so the FP32 cull may take its
+                                  common-origin form (option "common_origin"; a batch of views only when every view is pinhole or
+                                  aperture 0 and all origins are equal bit for bit)                                           */
     RT_CTR_COUNT = 24
 };
 
@@ -290,6 +293,35 @@ int rt_render_accumulate_device(rt_ctx* ctx, int nx, int ny, int sample_begin, i
  * d_rgb8 is a DEVICE pointer (nx*ny*3 bytes).                                                   */
 int rt_resolve_device(rt_ctx* ctx, int nx, int ny, int nsamples_total, const float* d_sum,
                       uint8_t* d_rgb8, void* stream, int sync);
+
+/* ---- batches of views (added within ABI version 2, like rt_get_bvh) ----------------------------
+ * Render n_views cameras of the current scene in one call: one pass of the chosen variant over a frame that stacks the
+ * n_views images (n_views * ny rows), so small frames fill the device together instead of one ramp-up and one tail each.
+ * View v renders exactly the paths that rt_set_camera(cam_types[v], cams + 24 v) + rt_render(nx, ny, nsamples, max_depth,
+ * seed, variant) renders (same Philox counters, bounces and radiance per path); only the order in which the device adds
+ * samples into the frame differs, so the float sums agree to their last bits and rgb8 to 1.
+ *   cam_types: n_views RT_CAM_*; cams: 24 * n_views floats, each an rt_set_camera record.  The cameras are per call:
+ *   the context's camera is neither needed nor changed.  An unknown type -> RT_ERR_UNSUPPORTED naming the view.
+ *   Limits (RT_ERR_ARG) are rt_render's on the stacked frame: n_views >= 1, n_views * nx * ny <= (2^31 - 1) / 3, samples
+ *   < 2^24, max_depth <= 255 for the wavefront variant.  A rejected call changes nothing of the context.
+ *   The movers' time window covers the union of the views' shutter intervals (views at different t0..t1 are the frames
+ *   of an animation).  Multi-device contexts partition the stacked frame as rt_render does (sample slices, or rows of
+ *   the stacked frame with option "rows" = 1).  RT_CTR_SAMPLES grows by n_views * nx * ny * nsamples.
+ *   out_linear_rgb / out_rgb8: n_views images, each in rt_render's layout, view v at offset v*nx*ny*3; either may be NULL. */
+int rt_render_views(rt_ctx* ctx, int n_views, const int32_t* cam_types, const float* cams,
+                    int nx, int ny, int nsamples, int max_depth, uint64_t seed, int variant,
+                    float* out_linear_rgb, uint8_t* out_rgb8);
+/* device-resident leg (torch / NCCL callers): += samples [sample_begin, sample_begin+sample_count) of every view into
+ * d_sum (DEVICE pointer on the context's first device, n_views*nx*ny*3 floats, view v at offset v*nx*ny*3), on `stream`
+ * after the work already enqueued there; returns after the kernels are enqueued if `sync` is 0.  A batch's cameras wait
+ * for the previous batch of the context, whatever its stream; the path queues and counters, as for
+ * rt_render_accumulate_device, assume that the device legs of one context are ordered (one stream, or sync = 1).      */
+int rt_render_views_accumulate_device(rt_ctx* ctx, int n_views, const int32_t* cam_types, const float* cams,
+                                      int nx, int ny, int sample_begin, int sample_count, int max_depth, uint64_t seed,
+                                      int variant, float* d_sum, void* stream, int sync);
+/* rt_resolve_device for n_views stacked images: each view y-flipped on its own (d_rgb8: n_views*nx*ny*3 bytes)          */
+int rt_resolve_views_device(rt_ctx* ctx, int n_views, int nx, int ny, int nsamples_total, const float* d_sum,
+                            uint8_t* d_rgb8, void* stream, int sync);
 
 /* ---- diagnostics used by the parity tests ---------------------------------------------- */
 

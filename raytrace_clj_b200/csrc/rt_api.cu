@@ -60,7 +60,10 @@ struct DeviceBuffers {
     float* d_sum = nullptr;
     float* d_mean = nullptr;
     uint8_t* d_rgb8 = nullptr;
-    size_t frame_px = 0;
+    size_t frame_px = 0;                  // pixels of the stacked frame the buffers hold (every view of rt_render_views)
+    DevCamera* d_views = nullptr;         // rt_render_views: the batch's cameras (grown on demand)
+    int views_cap = 0;
+    cudaEvent_t ev_views = nullptr;       // recorded after the last batch that read d_views: the next upload waits for it
     unsigned long long* d_counters = nullptr;   // DC_COUNT + 1 (last = work counter)
     // wavefront queues
     struct WaveLane {
@@ -185,6 +188,7 @@ struct rt_ctx {
     bool profile = false;
     double stage_ms[4] = {0, 0, 0, 0};   // cull, refine, tie-break, shade (profile mode)
     double reduce_ms = 0.0;              // cross-device reduce of the multi-device renders since the last reset
+    uint64_t common_origin_rays = 0;     // RT_CTR_COMMON_ORIGIN_RAYS
     std::vector<bool> peer_ok;
     NcclApi nccl;
 };
@@ -351,9 +355,9 @@ Options options_from_env() {
 // Wavefront render of one device's share: enqueue iterations (cull, refine, shade) ahead of the
 // GPU and poll the queue count every kWaveChunk iterations; returns when the queue has drained (the last
 // polled chunk may still be finishing its empty kernels).
-template <int BLOCK, int MINB>
+template <int BLOCK, int MINB, bool VIEWS>
 int cull_config(rt_ctx* ctx, size_t* smem, int* bps, void (**kern)(const WaveParams)) {
-    *kern = wf_cull<kR, BLOCK, MINB>;
+    *kern = wf_cull<kR, BLOCK, MINB, VIEWS>;
     // a resident scene keeps two tiles (general + common-origin records); a tiled scene streams ONE tile and the loader
     // writes whichever form the batch needs
     *smem = (ctx->preloaded ? 2 : 1) * (size_t)ctx->cull_cap * sizeof(float4) + Culler<kR, BLOCK>::LIST_BYTES;
@@ -361,6 +365,29 @@ int cull_config(rt_ctx* ctx, size_t* smem, int* bps, void (**kern)(const WavePar
     RT_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(bps, *kern, BLOCK, *smem));
     if (*bps < 1) return fail(ctx, RT_ERR_CUDA, "cull kernel does not fit on an SM");
     return RT_OK;
+}
+
+// The stage kernels of one wavefront render.  VIEWS = true: the instantiations a batch of views (rt_render_views) runs; the
+// single-camera ones (false) hold none of the batch code, so a single render runs exactly the kernels it ran before batches.
+struct StageKernels {
+    void (*tail)(const WaveParams);
+    void (*refine)(const WaveParams);
+    void (*shade)(const WaveParams);
+    void (*bvh)(const WaveParams);
+    void (*cull_tc)(const WaveParams);
+};
+template <bool VIEWS>
+StageKernels stage_kernels(bool gen, bool tail4, int tail_block) {
+    StageKernels k;
+    k.tail = gen ? wf_tail<256, true, 1, VIEWS> : (tail4 ? wf_tail<256, false, 4, VIEWS> : wf_tail<256, false, 1, VIEWS>);
+    if (tail_block == 128) k.tail = wf_tail<128, false, 1, VIEWS>;
+    if (tail_block == 64) k.tail = wf_tail<64, false, 1, VIEWS>;
+    if (tail_block == 32) k.tail = wf_tail<32, false, 1, VIEWS>;
+    k.refine = gen ? wf_refine<true, VIEWS> : wf_refine<false, VIEWS>;
+    k.shade = gen ? wf_shade<true, VIEWS> : wf_shade<false, VIEWS>;
+    k.bvh = gen ? wf_bvh<true, VIEWS> : wf_bvh<false, VIEWS>;
+    k.cull_tc = wf_cull_tc<VIEWS>;
+    return k;
 }
 
 // Wavefront render of one device's share.  The path population is split into `lanes` independent halves,
@@ -375,9 +402,15 @@ int launch_wave(rt_ctx* ctx, DeviceBuffers& d, const RenderParams& P, unsigned l
     void (*cull)(const WaveParams) = nullptr;
     size_t smem = 0;
     int bps = 0, cull_block = 256, rc;
-    if (opt.cull_shape == 2) rc = cull_config<256, 2>(ctx, &smem, &bps, &cull);
-    else if (opt.cull_shape == 1) { rc = cull_config<128, 6>(ctx, &smem, &bps, &cull); cull_block = 128; }
-    else { rc = cull_config<128, 5>(ctx, &smem, &bps, &cull); cull_block = 128; }
+    // a batch of views (rt_render_views) runs its own instantiation of the cull; shape 1's register cap (80) does not hold
+    // the view's camera, so such a batch runs shape 0
+    const bool views = P.views != nullptr;
+    if (opt.cull_shape == 2) rc = views ? cull_config<256, 2, true>(ctx, &smem, &bps, &cull) : cull_config<256, 2, false>(ctx, &smem, &bps, &cull);
+    else if (opt.cull_shape == 1 && !views) { rc = cull_config<128, 6, false>(ctx, &smem, &bps, &cull); cull_block = 128; }
+    else {
+        rc = views ? cull_config<128, 5, true>(ctx, &smem, &bps, &cull) : cull_config<128, 5, false>(ctx, &smem, &bps, &cull);
+        cull_block = 128;
+    }
     if (rc) return rc;
     const int cull_ctas_env = opt.cull_ctas_per_sm;                       // one fewer than the occupancy limit leaves
     if (cull_ctas_env > 0) bps = std::min(bps, cull_ctas_env);           // room for the other lane's light kernels
@@ -398,19 +431,17 @@ int launch_wave(rt_ctx* ctx, DeviceBuffers& d, const RenderParams& P, unsigned l
     const size_t tail_smem = (size_t)ctx->cull_cap * sizeof(float4) +
                              (tail4 ? Culler<4, 256>::LIST_BYTES : (size_t)Culler<1, 256>::LIST_WORDS * tail_block * sizeof(uint32_t));
     int tail_bps = 0;
-    void (*k_tail)(const WaveParams) = gen ? wf_tail<256, true, 1> : (tail4 ? wf_tail<256, false, 4> : wf_tail<256, false, 1>);
-    if (tail_block == 128) k_tail = wf_tail<128, false, 1>;
-    if (tail_block == 64) k_tail = wf_tail<64, false, 1>;
-    if (tail_block == 32) k_tail = wf_tail<32, false, 1>;
-    void (*k_refine)(const WaveParams) = gen ? wf_refine<true> : wf_refine<false>;
-    void (*k_shade)(const WaveParams) = gen ? wf_shade<true> : wf_shade<false>;
+    const StageKernels K = views ? stage_kernels<true>(gen, tail4, tail_block) : stage_kernels<false>(gen, tail4, tail_block);
+    void (*k_tail)(const WaveParams) = K.tail;
+    void (*k_refine)(const WaveParams) = K.refine;
+    void (*k_shade)(const WaveParams) = K.shade;
     RT_CUDA(ctx, cudaFuncSetAttribute(k_tail, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tail_smem));
     RT_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&tail_bps, k_tail, tail_block, tail_smem));
     // automatic: the same number of tail THREADS per SM whatever the CTA size (256 per lane with two lanes, 512 with one)
     const int tail_auto = (n_lanes > 1 ? 1 : std::max(1, std::min((int)(tail_bps * tail_block / 256), 2))) * (256 / tail_block);
     const int tail_grid = d.sm_count * (opt.tail_ctas_per_sm > 0 ? opt.tail_ctas_per_sm : tail_auto);
     const bool bvh = ctx->accel == RT_ACCEL_BVH;   // closest hit through the tree: one wf_bvh launch instead of cull + refine + tie-break
-    void (*k_bvh)(const WaveParams) = gen ? wf_bvh<true> : wf_bvh<false>;
+    void (*k_bvh)(const WaveParams) = K.bvh;
     const bool tail_ok = tail_bps >= 1 && tail_entries > 0 && !ctx->profile && !bvh;
     // tensor-core cull (rt_cull_tc.cuh): one 544-thread CTA per SM, the whole sphere-feature list resident in shared memory
     // (below ~160 leaves most of a 256-column feature tile is padding and the FP32 loop wins: C5-100 39.7 vs 48.0 ms, Cornell box
@@ -422,7 +453,7 @@ int launch_wave(rt_ctx* ctx, DeviceBuffers& d, const RenderParams& P, unsigned l
     const int tc_launch_tiles = std::min(ctx->tc_tiles, (int)tc::MAX_TILES);
     const int tc_slots = tc::slots_for(tc_launch_tiles, 227 * 1024);
     const size_t tc_smem = tc::smem_bytes(tc_launch_tiles, tc_slots);
-    if (use_tc) RT_CUDA(ctx, cudaFuncSetAttribute(wf_cull_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem));
+    if (use_tc) RT_CUDA(ctx, cudaFuncSetAttribute(K.cull_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem));
     const int tc_per_cta = std::max(0, opt.tc_tiles_per_cta);
     const int tc_grid = opt.tc_ctas > 0 ? std::min(opt.tc_ctas, 4 * d.sm_count) : d.sm_count;
     // one launch per 1024 leaves of the list ("pass"): the pairs of all passes pile up in the same buffer
@@ -434,7 +465,7 @@ int launch_wave(rt_ctx* ctx, DeviceBuffers& d, const RenderParams& P, unsigned l
             Wt.tc_tile0 = t0;
             Wt.tc_launch_tiles = std::min((int)tc::MAX_TILES, ctx->tc_tiles - t0);
             Wt.tc_pass = pass;
-            wf_cull_tc<<<ctas, tc::THREADS, tc_smem, s_>>>(Wt);
+            K.cull_tc<<<ctas, tc::THREADS, tc_smem, s_>>>(Wt);
             if (pass) ctx->n_launches += 1;
         }
     };
@@ -691,19 +722,60 @@ int launch_wave(rt_ctx* ctx, DeviceBuffers& d, const RenderParams& P, unsigned l
 
 int launch_params(rt_ctx* ctx, DeviceBuffers& d, RenderParams& P, int variant, cudaStream_t stream);
 
-// Launch the render kernels for one device's share of the work (async on d.stream).
-int launch_render(rt_ctx* ctx, DeviceBuffers& d, int nx, int ny, int sample_begin, int sample_count, int row_offset,
-                  int row_stride, int max_depth, uint64_t seed, int variant, float* d_sum, cudaStream_t stream) {
+// every camera ray of these cameras starts at cams[0].origin: pinhole or aperture 0, and one origin bit for bit (a cube map)
+bool cameras_share_origin(const DevCamera* cams, int n_views) {
+    for (int v = 0; v < n_views; ++v) {
+        const DevCamera& c = cams[v];
+        if (!(c.type == CAM_PINHOLE || c.lens_radius == 0.f)) return false;
+        if (memcmp(&c.origin, &cams[0].origin, sizeof(float3)) != 0) return false;
+    }
+    return true;
+}
+
+// Launch the render kernels for one device's share of the work (async on `stream`): n_views cameras (host records; 1 =
+// a single render, whose camera travels in the parameters) over a frame of n_views stacked nx x ny images, rows
+// row_offset + k row_stride of the stacked frame.
+int launch_render(rt_ctx* ctx, DeviceBuffers& d, const DevCamera* cams, int n_views, int nx, int ny, int sample_begin,
+                  int sample_count, int row_offset, int row_stride, int max_depth, uint64_t seed, int variant, float* d_sum,
+                  cudaStream_t stream) {
     RenderParams P{};
     P.sc = d.sc;
-    P.cam = ctx->cam;
+    P.cam = cams[0];
+    P.common_origin = cameras_share_origin(cams, n_views) ? 1 : 0;
+    if (n_views > 1) {
+        // the table is one per device: a batch on another stream (rt_render_views_accumulate_device with sync = 0) may
+        // still read it, so the upload waits for the last batch that did
+        if (!d.ev_views) RT_CUDA(ctx, cudaEventCreateWithFlags(&d.ev_views, cudaEventDisableTiming));
+        else RT_CUDA(ctx, cudaStreamWaitEvent(stream, d.ev_views, 0));
+        if (d.views_cap < n_views) {
+            if (d.d_views) { RT_CUDA(ctx, cudaEventSynchronize(d.ev_views)); cudaFree(d.d_views); }
+            d.d_views = nullptr;
+            d.views_cap = 0;
+            RT_CUDA(ctx, cudaMalloc(&d.d_views, (size_t)n_views * sizeof(DevCamera)));
+            d.views_cap = n_views;
+        }
+        RT_CUDA(ctx, cudaMemcpyAsync(d.d_views, cams, (size_t)n_views * sizeof(DevCamera), cudaMemcpyHostToDevice, stream));
+        // slot / view_px as a multiply-high (view_of): with s = ceil(log2 view_px) and magic = ceil(2^(31+s) / view_px)
+        // (< 2^32), umulhi(2 slot, magic) >> s = floor(slot magic / 2^(31+s)) is exact for every slot below 2^31 (the
+        // stacked frame has fewer than 2^31 / 3): the rounding up of magic adds less than slot / 2^(31+s) < 1 / view_px.
+        const uint64_t px = (uint64_t)nx * (uint64_t)ny;
+        uint32_t s = 0;
+        while ((1ull << s) < px) ++s;
+        P.views = d.d_views;
+        P.n_views = n_views;
+        P.view_px = (uint32_t)px;
+        P.view_mask = (uint32_t)((1ull << s) - 1);   // a tag (v << s) | pixel stays below 2^31: v 2^s < 2 n_views view_px
+        P.view_bits = s;
+        P.view_magic = (uint32_t)(((1ull << (31 + s)) + px - 1) / px);
+        P.view_shift = s;
+    }
     P.nx = nx;
     P.ny = ny;
     P.sample_begin = sample_begin;
     P.sample_count = sample_count;
     P.row_offset = row_offset;
     P.row_stride = row_stride;
-    P.rows_in_shard = (ny - row_offset + row_stride - 1) / row_stride;
+    P.rows_in_shard = (n_views * ny - row_offset + row_stride - 1) / row_stride;
     P.max_depth = max_depth;
     P.key = make_uint2((uint32_t)seed, (uint32_t)(seed >> 32));
     P.sum = d_sum;
@@ -711,22 +783,28 @@ int launch_render(rt_ctx* ctx, DeviceBuffers& d, int nx, int ny, int sample_begi
     P.work_counter = d.d_counters + DC_COUNT;
     P.total_work = (unsigned long long)sample_count * (unsigned long long)nx * (unsigned long long)P.rows_in_shard;
     if ((sample_begin + sample_count) >= (1 << 24)) return fail(ctx, RT_ERR_ARG, "sample index must stay below 2^24");
-    return launch_params(ctx, d, P, variant, stream);
+    int rc = launch_params(ctx, d, P, variant, stream);
+    if (rc == RT_OK && n_views > 1) RT_CUDA(ctx, cudaEventRecord(d.ev_views, stream));   // the wavefront lanes join `stream` first
+    return rc;
 }
 
-// P: scene-independent fields filled by the caller (frame, work, seed, outputs); the rest is completed here
+// P: scene-independent fields filled by the caller (frame, cameras, work, seed, outputs); the rest is completed here
 int launch_params(rt_ctx* ctx, DeviceBuffers& d, RenderParams& P, int variant, cudaStream_t stream) {
     if (variant != RT_VARIANT_MEGAKERNEL && variant != RT_VARIANT_WAVEFRONT)
         return fail(ctx, RT_ERR_ARG, "unknown render variant");
     if (variant == RT_VARIANT_WAVEFRONT && P.max_depth > 255)
         return fail(ctx, RT_ERR_ARG, "the wavefront variant packs the depth in 8 bits: max_depth <= 255");
     P.sc = d.sc;
-    P.cam = ctx->cam;
     P.counters = d.d_counters;
     P.work_counter = d.d_counters + DC_COUNT;
     P.cull_cap = ctx->cull_cap;
     P.preloaded = ctx->preloaded;
-    P.common_origin = (ctx->opt.common_origin && (ctx->cam.type == CAM_PINHOLE || ctx->cam.lens_radius == 0.f)) ? 1 : 0;
+    P.common_origin = (ctx->opt.common_origin && P.common_origin) ? 1 : 0;   // the caller: the cameras share an origin
+    if (!P.views) {   // one camera: a queue record's tag is its frame slot
+        P.view_mask = ~0u;
+        P.view_bits = 31;
+        P.view_px = 0;
+    }
     RT_CUDA(ctx, cudaMemsetAsync(P.work_counter, 0, sizeof(unsigned long long), stream));
     if (P.total_work == 0) return RT_OK;
     size_t smem = mega_smem_bytes(ctx->cull_cap);
@@ -737,6 +815,8 @@ int launch_params(rt_ctx* ctx, DeviceBuffers& d, RenderParams& P, int variant, c
         // reproducibility check (tests/test_gpu_parity.py::test_render_is_reproducible runs both)
         void (*kern)(const RenderParams) = ctx->generic ? mega_kernel<kR, kBlock, kMinBlocks, true>
                                            : (ctx->opt.mega_regcap ? mega_kernel<kR, kBlock, 2, false> : mega_kernel<kR, kBlock, kMinBlocks, false>);
+        if (P.views)   // a batch of views: the uncapped build only (the register-capped A/B build has no batch form)
+            kern = ctx->generic ? mega_views_kernel<kR, kBlock, kMinBlocks, true> : mega_views_kernel<kR, kBlock, kMinBlocks, false>;
         int rc = configure_kernel(ctx, kern, smem, &bps);
         if (rc) return rc;
         int grid = (int)std::min<unsigned long long>((unsigned long long)d.sm_count * bps, want);
@@ -747,6 +827,7 @@ int launch_params(rt_ctx* ctx, DeviceBuffers& d, RenderParams& P, int variant, c
         return RT_OK;
     }
     // persistent wavefront: every CTA is an independent engine with its own queues
+    if (P.common_origin) ctx->common_origin_rays += P.total_work;
     return launch_wave(ctx, d, P, want, stream);
 }
 
@@ -1158,6 +1239,233 @@ int check_camera_times(rt_ctx* ctx) {
     return ctx->accel == RT_ACCEL_BVH ? ensure_bvh(ctx) : RT_OK;
 }
 
+// the kernels' form of one rt_set_camera record (camera.clj:35-48)
+DevCamera make_camera(int cam_type, const float* cam) {
+    DevCamera c{};
+    c.type = cam_type;
+    auto g = [&](int k) { return make_float3(cam[3 * k], cam[3 * k + 1], cam[3 * k + 2]); };
+    c.origin = g(0); c.lleft = g(1); c.horiz = g(2); c.vert = g(3); c.u = g(4); c.v = g(5); c.w = g(6);
+    c.lens_radius = cam[21] / 2.0f;   // camera.clj:38
+    c.t0 = cam[22];
+    c.t1 = cam[23];
+    return c;
+}
+
+// The cameras of an rt_render_views call, each checked as rt_set_camera checks one, plus a finite shutter interval.
+int marshal_views(rt_ctx* ctx, int n_views, const int32_t* cam_types, const float* cams, std::vector<DevCamera>& out) {
+    out.resize((size_t)n_views);
+    for (int v = 0; v < n_views; ++v) {
+        if (cam_types[v] != RT_CAM_PINHOLE && cam_types[v] != RT_CAM_THIN_LENS)
+            return fail(ctx, RT_ERR_UNSUPPORTED, "view " + std::to_string(v) + ": unknown camera type");
+        out[(size_t)v] = make_camera(cam_types[v], cams + (size_t)24 * v);
+        if (cam_types[v] == RT_CAM_THIN_LENS && !(std::isfinite(out[(size_t)v].t0) && std::isfinite(out[(size_t)v].t1)))
+            return fail(ctx, RT_ERR_ARG, "view " + std::to_string(v) + ": ray time is not finite");
+    }
+    return RT_OK;
+}
+
+// Checks of an rt_render_views call that need no device work, so that a rejected call changes nothing: the limits of
+// rt_render on the stacked frame of n_views images, then the cameras.
+int check_views(rt_ctx* ctx, int n_views, const int32_t* cam_types, const float* cams, int nx, int ny, int sample_end,
+                int max_depth, int variant, std::vector<DevCamera>& out) {
+    if (n_views < 1 || !cam_types || !cams || nx <= 0 || ny <= 0 || max_depth < 0)
+        return fail(ctx, RT_ERR_ARG, "bad render_views arguments");
+    if ((long long)nx * ny > 0x7fffffffLL / 3 || (long long)nx * ny * n_views > 0x7fffffffLL / 3)
+        return fail(ctx, RT_ERR_ARG, "image too large: n_views * nx * ny must stay within (2^31 - 1) / 3");
+    if (sample_end >= (1 << 24)) return fail(ctx, RT_ERR_ARG, "sample index must stay below 2^24");
+    if (variant != RT_VARIANT_MEGAKERNEL && variant != RT_VARIANT_WAVEFRONT) return fail(ctx, RT_ERR_ARG, "unknown render variant");
+    if (variant == RT_VARIANT_WAVEFRONT && max_depth > 255)
+        return fail(ctx, RT_ERR_ARG, "the wavefront variant packs the depth in 8 bits: max_depth <= 255");
+    return marshal_views(ctx, n_views, cam_types, cams, out);
+}
+
+// check_camera_times for a batch: the movers' window covers the union of the views' shutter intervals
+int prepare_views(rt_ctx* ctx, const std::vector<DevCamera>& views) {
+    double lo = 0.0, hi = 0.0;
+    for (size_t v = 0; v < views.size(); ++v) {
+        const DevCamera& c = views[v];
+        const double a = c.type == CAM_THIN_LENS ? std::min(c.t0, c.t1) : 0.0, b = c.type == CAM_THIN_LENS ? std::max(c.t0, c.t1) : 0.0;
+        lo = v ? std::min(lo, a) : a;
+        hi = v ? std::max(hi, b) : b;
+    }
+    if (int rc = ensure_window(ctx, lo, hi)) return rc;
+    return ctx->accel == RT_ACCEL_BVH ? ensure_bvh(ctx) : RT_OK;
+}
+
+// rt_render for n_views cameras over one stacked frame (rt_render: the context's camera, n_views = 1).  The caller has
+// checked the arguments and prepared the cameras' time window.
+int render_frames(rt_ctx* ctx, const DevCamera* cams, int n_views, int nx, int ny, int nsamples, int max_depth, uint64_t seed,
+                  int variant, float* out_linear_rgb, uint8_t* out_rgb8) {
+    int rc = RT_OK;
+    const size_t px = (size_t)nx * ny * n_views;   // every view: the frame slot of view v's pixel (i, j) is (v ny + j) nx + i
+    const int G = (int)ctx->devs.size();
+    const bool by_rows = G > 1 && ctx->opt.rows != 0;
+    const bool use_nccl = G > 1 && ctx->opt.reduce != 0;
+    if (use_nccl && (rc = ensure_nccl(ctx))) return rc;
+    // Partition over the devices of the context (core.clj:100-108's chunk pool, SURVEY 8e): sample slices — device g
+    // renders samples [g*S/G, (g+1)*S/G) of every pixel — or interleaved rows — device g renders rows j = g (mod G) of the
+    // stacked frame with all S samples.  One host thread per device (each feeds its own wavefront loop).
+    auto device_work = [&](int g) -> int {
+        DeviceBuffers& d = ctx->devs[g];
+        RT_CUDA(ctx, cudaSetDevice(d.dev));
+        int r = ensure_frame(ctx, d, px);
+        if (r) return r;
+        int s0 = (int)((long long)nsamples * g / G), s1 = (int)((long long)nsamples * (g + 1) / G);
+        RT_CUDA(ctx, cudaEventRecord(d.ev0, d.stream));
+        RT_CUDA(ctx, cudaMemsetAsync(d.d_sum, 0, px * 3 * sizeof(float), d.stream));
+        if (by_rows) r = launch_render(ctx, d, cams, n_views, nx, ny, 0, nsamples, g, G, max_depth, seed, variant, d.d_sum, d.stream);
+        else r = launch_render(ctx, d, cams, n_views, nx, ny, s0, s1 - s0, 0, 1, max_depth, seed, variant, d.d_sum, d.stream);
+        if (r) return r;
+        RT_CUDA(ctx, cudaEventRecord(d.ev1, d.stream));
+        RT_CUDA(ctx, cudaEventRecord(d.ev_done, d.stream));
+        d.timed = true;
+        return RT_OK;
+    };
+    if (G == 1) {
+        if ((rc = device_work(0))) return rc;
+    } else {
+        std::vector<int> rcs((size_t)G, RT_OK);
+        std::vector<std::thread> workers;
+        for (int g = 0; g < G; ++g) workers.emplace_back([&, g] { rcs[(size_t)g] = device_work(g); });
+        for (auto& w : workers) w.join();
+        int bad = RT_OK;
+        for (int g = 0; g < G; ++g)
+            if (rcs[(size_t)g] && !bad) bad = rcs[(size_t)g];
+        if (bad) {   // the other devices may still be rendering into buffers the next call reuses: drain them first
+            for (auto& dv : ctx->devs) { cudaSetDevice(dv.dev); cudaDeviceSynchronize(); }
+            cudaSetDevice(ctx->devs[0].dev);
+            return bad;
+        }
+    }
+    // combine on the root device.  Default: the resolve kernel reads the peers' float sums over NVLink peer mappings (the
+    // reduce fused into core.clj:52-57's gamma / quantise pass).  Option "reduce" = 1: one ncclReduce(sum, float32,
+    // nx*ny*3, root 0) over the per-device communicators, then the plain resolve.
+    DeviceBuffers& root = ctx->devs[0];
+    RT_CUDA(ctx, cudaSetDevice(root.dev));
+    ResolveParams P{};
+    P.sum = root.d_sum; P.n_peers = 0; P.nx = nx; P.ny = ny; P.nr = nsamples; P.n_views = n_views;
+    P.rgb8 = out_rgb8 ? root.d_rgb8 : nullptr;
+    P.mean = out_linear_rgb ? root.d_mean : nullptr;
+    P.sum_out = nullptr;
+    const int total = (int)px * 3;
+    if (use_nccl) {
+        NcclApi& N = ctx->nccl;
+        for (int g = 1; g < G; ++g) RT_CUDA(ctx, cudaStreamWaitEvent(root.stream, ctx->devs[g].ev_done, 0));   // time the reduce alone
+        RT_CUDA(ctx, cudaEventRecord(root.ev_r0, root.stream));
+        ncclResult_t nr = N.GroupStart();
+        for (int g = 0; g < G && nr == ncclSuccess; ++g)
+            nr = N.Reduce(ctx->devs[g].d_sum, ctx->devs[g].d_sum, (size_t)total, ncclFloat, ncclSum, 0, N.comms[(size_t)g], ctx->devs[g].stream);
+        const ncclResult_t ge = N.GroupEnd();
+        if (nr == ncclSuccess) nr = ge;
+        if (nr != ncclSuccess) {
+            for (auto& dv : ctx->devs) { cudaSetDevice(dv.dev); cudaDeviceSynchronize(); }
+            cudaSetDevice(root.dev);
+            return fail(ctx, RT_ERR_NCCL, std::string("ncclReduce: ") + N.GetErrorString(nr));
+        }
+        RT_CUDA(ctx, cudaSetDevice(root.dev));
+        RT_CUDA(ctx, cudaEventRecord(root.ev_r1, root.stream));
+        resolve_kernel<<<(total + 255) / 256, 256, 0, root.stream>>>(P);
+    } else {
+        for (int g = 1; g < G; ++g) {
+            DeviceBuffers& d = ctx->devs[g];
+            RT_CUDA(ctx, cudaStreamWaitEvent(root.stream, d.ev_done, 0));
+            if (ctx->peer_ok[g]) {
+                P.peers[P.n_peers++] = d.d_sum;
+            } else {   // no peer mapping: stage through a copy, then add
+                if ((rc = ensure_scratch(ctx, root, (size_t)(G - 1) * px * 3 * sizeof(float)))) return rc;
+                float* stage = (float*)root.scratch + (size_t)(g - 1) * px * 3;
+                RT_CUDA(ctx, cudaMemcpyPeerAsync(stage, root.dev, d.d_sum, d.dev, px * 3 * sizeof(float), root.stream));
+                P.peers[P.n_peers++] = stage;
+            }
+        }
+        RT_CUDA(ctx, cudaEventRecord(root.ev_r0, root.stream));
+        resolve_kernel<<<(total + 255) / 256, 256, 0, root.stream>>>(P);   // reduce + resolve in one pass
+        RT_CUDA(ctx, cudaEventRecord(root.ev_r1, root.stream));
+    }
+    RT_CUDA(ctx, cudaGetLastError());
+    ctx->n_launches += 1;
+    // results: D2H into pinned staging at link speed, then one host memcpy into the caller's (pageable) buffer
+    auto host_pinned = [](const void* p) {
+        cudaPointerAttributes at{};
+        if (cudaPointerGetAttributes(&at, p) != cudaSuccess) { cudaGetLastError(); return false; }
+        return at.type == cudaMemoryTypeHost;
+    };
+    const size_t b_lin = out_linear_rgb ? align_up(px * 3 * sizeof(float), 256) : 0, b_rgb = out_rgb8 ? px * 3 : 0;
+    if (b_lin + b_rgb) {
+        if ((rc = ensure_stage(ctx, root, b_lin + b_rgb))) return rc;
+        constexpr int NCH = 4;
+        for (auto& e : root.ev_chunk)
+            if (!e) RT_CUDA(ctx, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+        struct Part { char* dst; const char* src; char* stage; size_t bytes; };
+        const Part parts[2] = {{(char*)out_linear_rgb, (const char*)root.d_mean, (char*)root.h_stage, out_linear_rgb ? px * 3 * sizeof(float) : 0},
+                               {(char*)out_rgb8, (const char*)root.d_rgb8, (char*)root.h_stage + b_lin, b_rgb}};
+        for (const Part& pt : parts) {
+            if (!pt.bytes) continue;
+            if (host_pinned(pt.dst)) {   // the caller's buffer is page-locked (rt_host_alloc / registered): the device writes it directly
+                RT_CUDA(ctx, cudaMemcpyAsync(pt.dst, pt.src, pt.bytes, cudaMemcpyDeviceToHost, root.stream));
+                continue;
+            }
+            const size_t step = align_up((pt.bytes + NCH - 1) / NCH, 4096);
+            for (int c = 0; c < NCH; ++c) {
+                const size_t off = std::min(pt.bytes, (size_t)c * step), len = std::min(pt.bytes - off, step);
+                if (len) RT_CUDA(ctx, cudaMemcpyAsync(pt.stage + off, pt.src + off, len, cudaMemcpyDeviceToHost, root.stream));
+                RT_CUDA(ctx, cudaEventRecord(root.ev_chunk[c], root.stream));
+            }
+            for (int c = 0; c < NCH; ++c) {
+                const size_t off = std::min(pt.bytes, (size_t)c * step), len = std::min(pt.bytes - off, step);
+                RT_CUDA(ctx, cudaEventSynchronize(root.ev_chunk[c]));
+                if (len) memcpy(pt.dst + off, pt.stage + off, len);
+            }
+        }
+    }
+    RT_CUDA(ctx, cudaStreamSynchronize(root.stream));
+    for (int g = 1; g < G; ++g) {
+        RT_CUDA(ctx, cudaSetDevice(ctx->devs[g].dev));
+        RT_CUDA(ctx, cudaStreamSynchronize(ctx->devs[g].stream));
+    }
+    cudaSetDevice(root.dev);
+    if (G > 1) {
+        float ms = 0.f;
+        if (cudaEventElapsedTime(&ms, root.ev_r0, root.ev_r1) == cudaSuccess) ctx->reduce_ms += ms;
+        cudaGetLastError();
+    }
+    return RT_OK;
+}
+
+// rt_render_accumulate_device for n_views cameras over one stacked frame, on the context's first device
+int accumulate_frames(rt_ctx* ctx, const DevCamera* cams, int n_views, int nx, int ny, int sample_begin, int sample_count,
+                      int row_offset, int row_stride, int max_depth, uint64_t seed, int variant, float* d_sum, void* stream,
+                      int sync) {
+    DeviceBuffers& d = ctx->devs[0];
+    RT_CUDA(ctx, cudaSetDevice(d.dev));
+    cudaStream_t st = (cudaStream_t)stream;
+    RT_CUDA(ctx, cudaEventRecord(d.ev0, st));
+    int rc = launch_render(ctx, d, cams, n_views, nx, ny, sample_begin, sample_count, row_offset, row_stride, max_depth, seed,
+                           variant, d_sum, st);
+    if (rc) return rc;
+    RT_CUDA(ctx, cudaEventRecord(d.ev1, st));
+    d.timed = true;
+    if (sync) RT_CUDA(ctx, cudaStreamSynchronize(st));
+    return RT_OK;
+}
+
+// rt_resolve_device for n_views stacked images
+int resolve_frames(rt_ctx* ctx, int n_views, int nx, int ny, int nsamples_total, const float* d_sum, uint8_t* d_rgb8,
+                   void* stream, int sync) {
+    DeviceBuffers& d = ctx->devs[0];
+    RT_CUDA(ctx, cudaSetDevice(d.dev));
+    ResolveParams P{};
+    P.sum = d_sum; P.n_peers = 0; P.nx = nx; P.ny = ny; P.nr = nsamples_total; P.n_views = n_views; P.rgb8 = d_rgb8;
+    P.mean = nullptr; P.sum_out = nullptr;
+    int total = nx * ny * n_views * 3;
+    cudaStream_t st = (cudaStream_t)stream;
+    resolve_kernel<<<(total + 255) / 256, 256, 0, st>>>(P);
+    RT_CUDA(ctx, cudaGetLastError());
+    ctx->n_launches += 1;
+    if (sync) RT_CUDA(ctx, cudaStreamSynchronize(st));
+    return RT_OK;
+}
+
 // Byte offsets of the scene blob's sections: one layout for rt_set_scene_ex and rt_set_scene_device, so that both write the
 // same bytes.  Every section starts on a 256-byte boundary and takes at least 16 bytes.
 struct SceneLayout {
@@ -1308,6 +1616,8 @@ void rt_destroy(rt_ctx* ctx) {
         if (d.d_sum) cudaFree(d.d_sum);
         if (d.d_mean) cudaFree(d.d_mean);
         if (d.d_rgb8) cudaFree(d.d_rgb8);
+        if (d.d_views) cudaFree(d.d_views);
+        if (d.ev_views) cudaEventDestroy(d.ev_views);
         if (d.d_counters) cudaFree(d.d_counters);
         if (d.scratch) cudaFree(d.scratch);
         free_wave(d);
@@ -2006,13 +2316,7 @@ int rt_set_camera(rt_ctx* ctx, int cam_type, const float cam[24]) {
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (!cam) return fail(ctx, RT_ERR_ARG, "cam is null");
     if (cam_type != RT_CAM_PINHOLE && cam_type != RT_CAM_THIN_LENS) return fail(ctx, RT_ERR_UNSUPPORTED, "unknown camera type");
-    DevCamera& c = ctx->cam;
-    c.type = cam_type;
-    auto g = [&](int k) { return make_float3(cam[3 * k], cam[3 * k + 1], cam[3 * k + 2]); };
-    c.origin = g(0); c.lleft = g(1); c.horiz = g(2); c.vert = g(3); c.u = g(4); c.v = g(5); c.w = g(6);
-    c.lens_radius = cam[21] / 2.0f;   // camera.clj:38
-    c.t0 = cam[22];
-    c.t1 = cam[23];
+    ctx->cam = make_camera(cam_type, cam);
     ctx->has_cam = true;
     return RT_OK;
 }
@@ -2028,16 +2332,8 @@ int rt_render_accumulate_device(rt_ctx* ctx, int nx, int ny, int sample_begin, i
         row_offset < 0 || row_offset >= row_stride)
         return fail(ctx, RT_ERR_ARG, "bad render arguments");
     if ((long long)nx * ny > 0x7fffffffLL / 3) return fail(ctx, RT_ERR_ARG, "image too large");
-    DeviceBuffers& d = ctx->devs[0];
-    RT_CUDA(ctx, cudaSetDevice(d.dev));
-    cudaStream_t st = (cudaStream_t)stream;
-    RT_CUDA(ctx, cudaEventRecord(d.ev0, st));
-    rc = launch_render(ctx, d, nx, ny, sample_begin, sample_count, row_offset, row_stride, max_depth, seed, variant, d_sum, st);
-    if (rc) return rc;
-    RT_CUDA(ctx, cudaEventRecord(d.ev1, st));
-    d.timed = true;
-    if (sync) RT_CUDA(ctx, cudaStreamSynchronize(st));
-    return RT_OK;
+    return accumulate_frames(ctx, &ctx->cam, 1, nx, ny, sample_begin, sample_count, row_offset, row_stride, max_depth, seed,
+                             variant, d_sum, stream, sync);
 }
 
 int rt_resolve_device(rt_ctx* ctx, int nx, int ny, int nsamples_total, const float* d_sum, uint8_t* d_rgb8, void* stream,
@@ -2045,17 +2341,7 @@ int rt_resolve_device(rt_ctx* ctx, int nx, int ny, int nsamples_total, const flo
     if (!ctx) return RT_ERR_ARG;
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (nx <= 0 || ny <= 0 || nsamples_total <= 0 || !d_sum || !d_rgb8) return fail(ctx, RT_ERR_ARG, "bad resolve arguments");
-    DeviceBuffers& d = ctx->devs[0];
-    RT_CUDA(ctx, cudaSetDevice(d.dev));
-    ResolveParams P{};
-    P.sum = d_sum; P.n_peers = 0; P.nx = nx; P.ny = ny; P.nr = nsamples_total; P.rgb8 = d_rgb8; P.mean = nullptr; P.sum_out = nullptr;
-    int total = nx * ny * 3;
-    cudaStream_t st = (cudaStream_t)stream;
-    resolve_kernel<<<(total + 255) / 256, 256, 0, st>>>(P);
-    RT_CUDA(ctx, cudaGetLastError());
-    ctx->n_launches += 1;
-    if (sync) RT_CUDA(ctx, cudaStreamSynchronize(st));
-    return RT_OK;
+    return resolve_frames(ctx, 1, nx, ny, nsamples_total, d_sum, d_rgb8, stream, sync);
 }
 
 int rt_render(rt_ctx* ctx, int nx, int ny, int nsamples, int max_depth, uint64_t seed, int variant, float* out_linear_rgb,
@@ -2066,139 +2352,44 @@ int rt_render(rt_ctx* ctx, int nx, int ny, int nsamples, int max_depth, uint64_t
     if ((rc = check_camera_times(ctx))) return rc;
     if (nx <= 0 || ny <= 0 || nsamples <= 0 || max_depth < 0) return fail(ctx, RT_ERR_ARG, "bad render arguments");
     if ((long long)nx * ny > 0x7fffffffLL / 3) return fail(ctx, RT_ERR_ARG, "image too large");
-    const size_t px = (size_t)nx * ny;
-    const int G = (int)ctx->devs.size();
-    const bool by_rows = G > 1 && ctx->opt.rows != 0;
-    const bool use_nccl = G > 1 && ctx->opt.reduce != 0;
-    if (use_nccl && (rc = ensure_nccl(ctx))) return rc;
-    // Partition over the devices of the context (core.clj:100-108's chunk pool, SURVEY 8e): sample slices — device g
-    // renders samples [g*S/G, (g+1)*S/G) of every pixel — or interleaved rows — device g renders rows j = g (mod G) with
-    // all S samples.  One host thread per device (each feeds its own wavefront loop).
-    auto device_work = [&](int g) -> int {
-        DeviceBuffers& d = ctx->devs[g];
-        RT_CUDA(ctx, cudaSetDevice(d.dev));
-        int r = ensure_frame(ctx, d, px);
-        if (r) return r;
-        int s0 = (int)((long long)nsamples * g / G), s1 = (int)((long long)nsamples * (g + 1) / G);
-        RT_CUDA(ctx, cudaEventRecord(d.ev0, d.stream));
-        RT_CUDA(ctx, cudaMemsetAsync(d.d_sum, 0, px * 3 * sizeof(float), d.stream));
-        if (by_rows) r = launch_render(ctx, d, nx, ny, 0, nsamples, g, G, max_depth, seed, variant, d.d_sum, d.stream);
-        else r = launch_render(ctx, d, nx, ny, s0, s1 - s0, 0, 1, max_depth, seed, variant, d.d_sum, d.stream);
-        if (r) return r;
-        RT_CUDA(ctx, cudaEventRecord(d.ev1, d.stream));
-        RT_CUDA(ctx, cudaEventRecord(d.ev_done, d.stream));
-        d.timed = true;
-        return RT_OK;
-    };
-    if (G == 1) {
-        if ((rc = device_work(0))) return rc;
-    } else {
-        std::vector<int> rcs((size_t)G, RT_OK);
-        std::vector<std::thread> workers;
-        for (int g = 0; g < G; ++g) workers.emplace_back([&, g] { rcs[(size_t)g] = device_work(g); });
-        for (auto& w : workers) w.join();
-        int bad = RT_OK;
-        for (int g = 0; g < G; ++g)
-            if (rcs[(size_t)g] && !bad) bad = rcs[(size_t)g];
-        if (bad) {   // the other devices may still be rendering into buffers the next call reuses: drain them first
-            for (auto& dv : ctx->devs) { cudaSetDevice(dv.dev); cudaDeviceSynchronize(); }
-            cudaSetDevice(ctx->devs[0].dev);
-            return bad;
-        }
-    }
-    // combine on the root device.  Default: the resolve kernel reads the peers' float sums over NVLink peer mappings (the
-    // reduce fused into core.clj:52-57's gamma / quantise pass).  Option "reduce" = 1: one ncclReduce(sum, float32,
-    // nx*ny*3, root 0) over the per-device communicators, then the plain resolve.
-    DeviceBuffers& root = ctx->devs[0];
-    RT_CUDA(ctx, cudaSetDevice(root.dev));
-    ResolveParams P{};
-    P.sum = root.d_sum; P.n_peers = 0; P.nx = nx; P.ny = ny; P.nr = nsamples;
-    P.rgb8 = out_rgb8 ? root.d_rgb8 : nullptr;
-    P.mean = out_linear_rgb ? root.d_mean : nullptr;
-    P.sum_out = nullptr;
-    const int total = nx * ny * 3;
-    if (use_nccl) {
-        NcclApi& N = ctx->nccl;
-        for (int g = 1; g < G; ++g) RT_CUDA(ctx, cudaStreamWaitEvent(root.stream, ctx->devs[g].ev_done, 0));   // time the reduce alone
-        RT_CUDA(ctx, cudaEventRecord(root.ev_r0, root.stream));
-        ncclResult_t nr = N.GroupStart();
-        for (int g = 0; g < G && nr == ncclSuccess; ++g)
-            nr = N.Reduce(ctx->devs[g].d_sum, ctx->devs[g].d_sum, (size_t)total, ncclFloat, ncclSum, 0, N.comms[(size_t)g], ctx->devs[g].stream);
-        const ncclResult_t ge = N.GroupEnd();
-        if (nr == ncclSuccess) nr = ge;
-        if (nr != ncclSuccess) {
-            for (auto& dv : ctx->devs) { cudaSetDevice(dv.dev); cudaDeviceSynchronize(); }
-            cudaSetDevice(root.dev);
-            return fail(ctx, RT_ERR_NCCL, std::string("ncclReduce: ") + N.GetErrorString(nr));
-        }
-        RT_CUDA(ctx, cudaSetDevice(root.dev));
-        RT_CUDA(ctx, cudaEventRecord(root.ev_r1, root.stream));
-        resolve_kernel<<<(total + 255) / 256, 256, 0, root.stream>>>(P);
-    } else {
-        for (int g = 1; g < G; ++g) {
-            DeviceBuffers& d = ctx->devs[g];
-            RT_CUDA(ctx, cudaStreamWaitEvent(root.stream, d.ev_done, 0));
-            if (ctx->peer_ok[g]) {
-                P.peers[P.n_peers++] = d.d_sum;
-            } else {   // no peer mapping: stage through a copy, then add
-                if ((rc = ensure_scratch(ctx, root, (size_t)(G - 1) * px * 3 * sizeof(float)))) return rc;
-                float* stage = (float*)root.scratch + (size_t)(g - 1) * px * 3;
-                RT_CUDA(ctx, cudaMemcpyPeerAsync(stage, root.dev, d.d_sum, d.dev, px * 3 * sizeof(float), root.stream));
-                P.peers[P.n_peers++] = stage;
-            }
-        }
-        RT_CUDA(ctx, cudaEventRecord(root.ev_r0, root.stream));
-        resolve_kernel<<<(total + 255) / 256, 256, 0, root.stream>>>(P);   // reduce + resolve in one pass
-        RT_CUDA(ctx, cudaEventRecord(root.ev_r1, root.stream));
-    }
-    RT_CUDA(ctx, cudaGetLastError());
-    ctx->n_launches += 1;
-    // results: D2H into pinned staging at link speed, then one host memcpy into the caller's (pageable) buffer
-    auto host_pinned = [](const void* p) {
-        cudaPointerAttributes at{};
-        if (cudaPointerGetAttributes(&at, p) != cudaSuccess) { cudaGetLastError(); return false; }
-        return at.type == cudaMemoryTypeHost;
-    };
-    const size_t b_lin = out_linear_rgb ? align_up(px * 3 * sizeof(float), 256) : 0, b_rgb = out_rgb8 ? px * 3 : 0;
-    if (b_lin + b_rgb) {
-        if ((rc = ensure_stage(ctx, root, b_lin + b_rgb))) return rc;
-        constexpr int NCH = 4;
-        for (auto& e : root.ev_chunk)
-            if (!e) RT_CUDA(ctx, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-        struct Part { char* dst; const char* src; char* stage; size_t bytes; };
-        const Part parts[2] = {{(char*)out_linear_rgb, (const char*)root.d_mean, (char*)root.h_stage, out_linear_rgb ? px * 3 * sizeof(float) : 0},
-                               {(char*)out_rgb8, (const char*)root.d_rgb8, (char*)root.h_stage + b_lin, b_rgb}};
-        for (const Part& pt : parts) {
-            if (!pt.bytes) continue;
-            if (host_pinned(pt.dst)) {   // the caller's buffer is page-locked (rt_host_alloc / registered): the device writes it directly
-                RT_CUDA(ctx, cudaMemcpyAsync(pt.dst, pt.src, pt.bytes, cudaMemcpyDeviceToHost, root.stream));
-                continue;
-            }
-            const size_t step = align_up((pt.bytes + NCH - 1) / NCH, 4096);
-            for (int c = 0; c < NCH; ++c) {
-                const size_t off = std::min(pt.bytes, (size_t)c * step), len = std::min(pt.bytes - off, step);
-                if (len) RT_CUDA(ctx, cudaMemcpyAsync(pt.stage + off, pt.src + off, len, cudaMemcpyDeviceToHost, root.stream));
-                RT_CUDA(ctx, cudaEventRecord(root.ev_chunk[c], root.stream));
-            }
-            for (int c = 0; c < NCH; ++c) {
-                const size_t off = std::min(pt.bytes, (size_t)c * step), len = std::min(pt.bytes - off, step);
-                RT_CUDA(ctx, cudaEventSynchronize(root.ev_chunk[c]));
-                if (len) memcpy(pt.dst + off, pt.stage + off, len);
-            }
-        }
-    }
-    RT_CUDA(ctx, cudaStreamSynchronize(root.stream));
-    for (int g = 1; g < G; ++g) {
-        RT_CUDA(ctx, cudaSetDevice(ctx->devs[g].dev));
-        RT_CUDA(ctx, cudaStreamSynchronize(ctx->devs[g].stream));
-    }
-    cudaSetDevice(root.dev);
-    if (G > 1) {
-        float ms = 0.f;
-        if (cudaEventElapsedTime(&ms, root.ev_r0, root.ev_r1) == cudaSuccess) ctx->reduce_ms += ms;
-        cudaGetLastError();
-    }
-    return RT_OK;
+    return render_frames(ctx, &ctx->cam, 1, nx, ny, nsamples, max_depth, seed, variant, out_linear_rgb, out_rgb8);
+}
+
+int rt_render_views(rt_ctx* ctx, int n_views, const int32_t* cam_types, const float* cams, int nx, int ny, int nsamples,
+                    int max_depth, uint64_t seed, int variant, float* out_linear_rgb, uint8_t* out_rgb8) {
+    int rc = check_ready(ctx);
+    if (rc) return rc;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    std::vector<DevCamera> views;
+    if (nsamples <= 0) return fail(ctx, RT_ERR_ARG, "bad render_views arguments");
+    if ((rc = check_views(ctx, n_views, cam_types, cams, nx, ny, nsamples, max_depth, variant, views))) return rc;
+    if ((rc = prepare_views(ctx, views))) return rc;
+    return render_frames(ctx, views.data(), n_views, nx, ny, nsamples, max_depth, seed, variant, out_linear_rgb, out_rgb8);
+}
+
+int rt_render_views_accumulate_device(rt_ctx* ctx, int n_views, const int32_t* cam_types, const float* cams, int nx, int ny,
+                                      int sample_begin, int sample_count, int max_depth, uint64_t seed, int variant,
+                                      float* d_sum, void* stream, int sync) {
+    int rc = check_ready(ctx);
+    if (rc) return rc;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    std::vector<DevCamera> views;
+    if (sample_begin < 0 || sample_count < 0 || !d_sum) return fail(ctx, RT_ERR_ARG, "bad render_views arguments");
+    if ((rc = check_views(ctx, n_views, cam_types, cams, nx, ny, sample_begin + sample_count, max_depth, variant, views))) return rc;
+    if ((rc = prepare_views(ctx, views))) return rc;
+    return accumulate_frames(ctx, views.data(), n_views, nx, ny, sample_begin, sample_count, 0, 1, max_depth, seed, variant,
+                             d_sum, stream, sync);
+}
+
+int rt_resolve_views_device(rt_ctx* ctx, int n_views, int nx, int ny, int nsamples_total, const float* d_sum, uint8_t* d_rgb8,
+                            void* stream, int sync) {
+    if (!ctx) return RT_ERR_ARG;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    if (n_views < 1 || nx <= 0 || ny <= 0 || nsamples_total <= 0 || !d_sum || !d_rgb8)
+        return fail(ctx, RT_ERR_ARG, "bad resolve arguments");
+    if ((long long)nx * ny > 0x7fffffffLL / 3 || (long long)nx * ny * n_views > 0x7fffffffLL / 3)
+        return fail(ctx, RT_ERR_ARG, "image too large: n_views * nx * ny must stay within (2^31 - 1) / 3");
+    return resolve_frames(ctx, n_views, nx, ny, nsamples_total, d_sum, d_rgb8, stream, sync);
 }
 
 int rt_host_alloc(rt_ctx* ctx, size_t bytes, void** out) {
@@ -2257,6 +2448,8 @@ int rt_trace_paths(rt_ctx* ctx, int nx, int ny, int n, const int32_t* pixel, con
         (d_log && (e = cudaMemsetAsync(d_log, 0xff, (size_t)n * log_bounces * sizeof(PathBounce), d.stream)) != cudaSuccess))
         return cleanup(fail(ctx, RT_ERR_CUDA, std::string("trace_paths upload: ") + cudaGetErrorString(e)));
     RenderParams P{};
+    P.cam = ctx->cam;
+    P.common_origin = cameras_share_origin(&ctx->cam, 1) ? 1 : 0;
     P.nx = nx; P.ny = ny;
     P.sample_begin = 0; P.sample_count = 1;
     P.row_offset = 0; P.row_stride = 1; P.rows_in_shard = ny;
@@ -2401,6 +2594,8 @@ int rt_cull_check(rt_ctx* ctx, int n, const float* origins, const float* dirs, c
         WaveParams W{};
         W.base.sc = d.sc;
         W.base.cam = ctx->cam;
+        W.base.view_mask = ~0u;
+        W.base.view_bits = 31;
         W.base.counters = d.d_counters;
         W.base.work_counter = d.d_counters + DC_COUNT;
         W.base.max_depth = 1;
@@ -2423,12 +2618,12 @@ int rt_cull_check(rt_ctx* ctx, int n, const float* origins, const float* dirs, c
         const int launch_tiles = std::min(ctx->tc_tiles, (int)tc::MAX_TILES);
         W.tc_slots = tc::slots_for(launch_tiles, 227 * 1024);
         const size_t tc_smem = tc::smem_bytes(launch_tiles, W.tc_slots);
-        RT_CUDA(ctx, cudaFuncSetAttribute(wf_cull_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem));
+        RT_CUDA(ctx, cudaFuncSetAttribute(wf_cull_tc<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem));
         for (int t0 = 0, pass = 0; t0 < ctx->tc_tiles; t0 += tc::MAX_TILES, ++pass) {
             W.tc_tile0 = t0;
             W.tc_launch_tiles = std::min((int)tc::MAX_TILES, ctx->tc_tiles - t0);
             W.tc_pass = pass;
-            wf_cull_tc<<<d.sm_count, tc::THREADS, tc_smem, d.stream>>>(W);
+            wf_cull_tc<false><<<d.sm_count, tc::THREADS, tc_smem, d.stream>>>(W);
         }
         tc_check_mark<<<d.sm_count * 4, 256, 0, d.stream>>>(W, d_mask, words);
         tc_check_compare<<<(n + 127) / 128, 128, 0, d.stream>>>(W, n, tmin, tmax, d_mask, words, d_out);
@@ -2611,6 +2806,7 @@ int rt_get_counters(rt_ctx* ctx, uint64_t out[RT_CTR_COUNT]) {
     out[RT_CTR_TIEBREAK_NS] = (uint64_t)(ctx->stage_ms[2] * 1e6);
     out[RT_CTR_SHADE_NS] = (uint64_t)(ctx->stage_ms[3] * 1e6);
     out[RT_CTR_REDUCE_NS] = (uint64_t)(ctx->reduce_ms * 1e6);
+    out[RT_CTR_COMMON_ORIGIN_RAYS] = ctx->common_origin_rays;
     return RT_OK;
 }
 
@@ -2626,6 +2822,7 @@ int rt_reset_counters(rt_ctx* ctx) {
     ctx->n_launches = 0;
     for (double& x : ctx->stage_ms) x = 0.0;
     ctx->reduce_ms = 0.0;
+    ctx->common_origin_rays = 0;
     return RT_OK;
 }
 

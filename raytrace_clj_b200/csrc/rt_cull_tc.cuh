@@ -214,6 +214,7 @@ __device__ __forceinline__ Smem carve(unsigned char* base, int tiles, int slots)
 
 // One ray of the tile: features into A[slot] (canonical layout), FP32 cull constants into ray[slot].
 // v = virtual queue index (v < n_g: path in flight, its record is loaded; else fresh: generated here and written).
+template <bool VIEWS>
 __device__ __forceinline__ void tc_produce_ray(const WaveParams& W, const tc::Smem& S, int slot, int rl, bool live, unsigned v, unsigned n_g,
                                                unsigned p0, unsigned long long gen_base, int cur) {
     const RenderParams& P = W.base;
@@ -231,7 +232,7 @@ __device__ __forceinline__ void tc_produce_ray(const WaveParams& W, const tc::Sm
             float4* q = qc + 3 * (size_t)(p0 + (v - n_g));
             TC_CHECK(p0 + (v - n_g) < (unsigned)W.capacity, "fresh entry", p0 + (v - n_g), W.capacity);
             TC_CHECK(gen_base + (v - n_g) < P.total_work, "work item", (unsigned)(gen_base + (v - n_g)), (unsigned)P.total_work);
-            make_path(P, gen_base + (v - n_g), a, b, c);
+            make_path<VIEWS>(P, gen_base + (v - n_g), a, b, c);
             q[0] = a; q[1] = b; q[2] = c;
         } else {
             TC_CHECK(v < (unsigned)W.capacity, "entry in flight", v, W.capacity);
@@ -383,6 +384,8 @@ __device__ __forceinline__ void tc_drain(const WaveParams& W, const tc::Smem& S,
 #define TC_T(var)
 #define TC_ACC(slot, since)
 #endif
+// VIEWS: instantiated for rt_render_views (false: single-camera renders)
+template <bool VIEWS>
 __global__ void __launch_bounds__(tc::THREADS, 1) wf_cull_tc(const __grid_constant__ WaveParams W) {
     TraceScope trace(W.trace);
     const RenderParams& P = W.base;
@@ -459,7 +462,7 @@ __global__ void __launch_bounds__(tc::THREADS, 1) wf_cull_tc(const __grid_consta
             TC_T(t2);
             if (it < n_it) {
                 const unsigned v = (first + it) * tc::TILE_M + rl;
-                tc_produce_ray(W, S, (int)s, (int)rl, v < n, v, n_g, p0, gen_base, W.cur);
+                tc_produce_ray<VIEWS>(W, S, (int)s, (int)rl, v < n, v, n_g, p0, gen_base, W.cur);
             }
             TC_ACC(2, t2);
             if (rl == 0) S.tile_of[s] = it < n_it ? (int)(first + it) : -1;

@@ -46,6 +46,16 @@ struct RenderParams {
     int cull_cap;                         // float4 slots of the shared-memory sphere tile
     int preloaded;                        // 1: whole scene fits one tile (loaded once per CTA)
     int common_origin;                    // 1: every camera ray starts at cam.origin (pinhole, or aperture 0)
+    // rt_render_views: the frame stacks n_views images of nx x ny; stacked row j_g is row j_g - v * ny of view
+    // v = j_g / ny, rendered through views[v] (P.cam = views[0]).  Null / 0 = the single camera in `cam`.
+    // A queue record's pixel field carries a TAG: the view-local Philox pixel in the low view_bits bits, the view above
+    // them, so that every bounce reads its Philox pixel with one AND (rng_pixel) and only the sample's RED.ADD rebuilds
+    // the frame slot (v * view_px + pixel, frame_slot).  A single render has view_mask = ~0, view_bits = 31, view_px = 0:
+    // the tag is the frame slot.  make_path splits a frame slot as umulhi(2 slot, view_magic) >> view_shift
+    // (= slot / view_px for every slot below 2^31).
+    const DevCamera* views;               // [n_views]
+    int n_views;
+    uint32_t view_px, view_mask, view_bits, view_magic, view_shift;   // view_px = nx * ny
     // rt_trace_paths: work item w IS path w of a caller-given list instead of the w-th (sample, pixel) of the frame;
     // the queue record's "pixel" field then holds w, `sum` has 3 floats per PATH, and the path's counters / bounce log
     // are kept per path.  All null / 0 in a render.
@@ -57,9 +67,21 @@ struct RenderParams {
     int path_log_n;
 };
 
-// the Philox "pixel" of the path whose queue record carries `slot` in its pixel field
-__device__ __forceinline__ uint32_t rng_pixel(const RenderParams& P, uint32_t slot) {
-    return P.path_pixel ? (uint32_t)__ldg(&P.path_pixel[slot]) : slot;
+// the view of a stacked frame slot (rt_render_views)
+__device__ __forceinline__ uint32_t view_of(const RenderParams& P, uint32_t slot) {
+    return __umulhi(slot << 1, P.view_magic) >> P.view_shift;
+}
+// the Philox "pixel" of the path whose queue record carries `tag` in its pixel field: a view's paths are keyed by the
+// view-local pixel, exactly as a single render of that camera keys them.  VIEWS = false (the instantiations that single
+// renders and rt_trace_paths run): the tag is the frame slot, and none of the batch arithmetic is compiled in.
+template <bool VIEWS>
+__device__ __forceinline__ uint32_t rng_pixel(const RenderParams& P, uint32_t tag) {
+    return P.path_pixel ? (uint32_t)__ldg(&P.path_pixel[tag]) : (VIEWS ? tag & P.view_mask : tag);
+}
+// the frame slot (the path of rt_trace_paths) a queue record's tag adds its radiance to
+template <bool VIEWS>
+__device__ __forceinline__ uint32_t frame_slot(const RenderParams& P, uint32_t tag) {
+    return VIEWS ? (tag & P.view_mask) + (tag >> P.view_bits) * P.view_px : tag;
 }
 // rt_trace_paths bookkeeping for ray number `ray_no` (0-based) of path `slot`
 __device__ __forceinline__ void path_log_ray(const RenderParams& P, uint32_t slot, int ray_no, float4 a, float4 b, int k, double t) {
@@ -529,7 +551,21 @@ __device__ __forceinline__ unsigned warp_claim(unsigned* counter, bool pred, uns
     return base + __popc(m & ((1u << lane) - 1u));
 }
 
-// camera ray of work item w as a queue record
+// rt_render_views: camera ray of view v's pixel (i, j) (view-local), out of line so that the single-camera path of the
+// kernels that generate rays keeps its registers
+struct CameraRay {
+    float3 o, d;
+    float time;
+};
+__device__ __noinline__ CameraRay view_ray(const DevCamera* __restrict__ views, uint32_t v, int nx, int ny, int i, int j,
+                                           uint32_t pixel, uint32_t sample, uint2 key) {
+    CameraRay r;
+    generate_ray(views[v], nx, ny, i, j, pixel, sample, key, r.o, r.d, r.time, nullptr);
+    return r;
+}
+
+// camera ray of work item w as a queue record.  VIEWS = false: a kernel instantiated for single-camera renders only.
+template <bool VIEWS>
 __device__ __forceinline__ void make_path(const RenderParams& P, unsigned long long w, float4& a, float4& b, float4& c) {
     const unsigned pshard = (unsigned)P.nx * (unsigned)P.rows_in_shard;
     unsigned s_local, q;
@@ -555,7 +591,15 @@ __device__ __forceinline__ void make_path(const RenderParams& P, unsigned long l
     }
     float3 o, d;
     float tmv;
-    generate_ray(P.cam, P.nx, P.ny, i, j, pix, smp, P.key, o, d, tmv, nullptr);
+    if (VIEWS && P.views && !P.path_pixel) {  // rt_render_views: the view's camera, view-local row and Philox pixel
+        const uint32_t v = view_of(P, slot);
+        pix = slot - v * P.view_px;
+        slot = pix | (v << P.view_bits);
+        const CameraRay r = view_ray(P.views, v, P.nx, P.ny, i, j - (int)v * P.ny, pix, smp, P.key);
+        o = r.o; d = r.d; tmv = r.time;
+    } else {
+        generate_ray(P.cam, P.nx, P.ny, i, j, pix, smp, P.key, o, d, tmv, nullptr);
+    }
     a = make_float4(o.x, o.y, o.z, tmv);
     b = make_float4(d.x, d.y, d.z, __uint_as_float(slot));
     c = make_float4(1.f, 1.f, 1.f, __uint_as_float((smp << 8) | (uint32_t)P.max_depth));
@@ -661,7 +705,7 @@ struct Scope {
     unsigned bid, nblk;
 };
 __device__ __forceinline__ Scope grid_scope() { return Scope{blockIdx.x, gridDim.x}; }
-template <int R, int BLOCK, bool COMMON>
+template <int R, int BLOCK, bool COMMON, bool VIEWS>
 __device__ __forceinline__ unsigned wf_cull_batches(const WaveParams& W, Scope sc_, int cur, unsigned e0, unsigned e1, unsigned n_g,
                                                     unsigned p0, unsigned long long gen0, int parts, unsigned item0, unsigned claimed,
                                                     int& budget, float4* s_cull, uint32_t* s_list) {
@@ -708,7 +752,7 @@ __device__ __forceinline__ unsigned wf_cull_batches(const WaveParams& W, Scope s
                 if (v >= n_g) {                               // fresh: generate the camera ray of its work item
                     float4 c;
                     float4* q = qc + 3 * (size_t)(p0 + (v - n_g));
-                    make_path(P, gen0 + (v - n_g), a, b, c);
+                    make_path<VIEWS>(P, gen0 + (v - n_g), a, b, c);
                     if (part == 0) { q[0] = a; q[1] = b; q[2] = c; }
                 } else {
                     a = qc[3 * (size_t)v];
@@ -734,7 +778,7 @@ __device__ __forceinline__ unsigned wf_cull_batches(const WaveParams& W, Scope s
 // batch apart — one-ray batches for the last stretch (two per warp of the grid), all claimed from the same counter.  A
 // short queue: 1 ray per thread, and below two batches per warp the sphere list is split across warps too (the pairs
 // merge in wf_refine).  R = 1 instantiates only the short form.  s_cullc may be null when n_p is 0 (the tail).
-template <int R, int BLOCK>
+template <int R, int BLOCK, bool VIEWS>
 __device__ __forceinline__ void wf_cull_body(const WaveParams& W, Scope sc_, int cur, unsigned n_g, unsigned n_p, unsigned long long gen_base,
                                              float4* s_cull, float4* s_cullc, uint32_t* s_list) {
     const RenderParams& P = W.base;
@@ -749,20 +793,20 @@ __device__ __forceinline__ void wf_cull_body(const WaveParams& W, Scope sc_, int
     const unsigned long long genC = gen_base - p0;   // C: virtual index = entry index; item = gen_base + (entry - p0)
     if (R > 1 && !P.preloaded) {
         // tiled scene: CTA-uniform static order; the tile loader builds the common-origin records itself
-        if (n_c) wf_cull_batches<R, BLOCK, true>(W, sc_, cur, p0, p0 + n_c, 0u, 0u, genC + 0u, 1, 0u, ITEM_NONE, budget, s_cull, s_list);
-        if (n_v) wf_cull_batches<R, BLOCK, false>(W, sc_, cur, 0u, n_v, n_g, p0, gen_base, 1, 0u, ITEM_NONE, budget, s_cull, s_list);
+        if (n_c) wf_cull_batches<R, BLOCK, true, VIEWS>(W, sc_, cur, p0, p0 + n_c, 0u, 0u, genC + 0u, 1, 0u, ITEM_NONE, budget, s_cull, s_list);
+        if (n_v) wf_cull_batches<R, BLOCK, false, VIEWS>(W, sc_, cur, 0u, n_v, n_g, p0, gen_base, 1, 0u, ITEM_NONE, budget, s_cull, s_list);
     } else if (R > 1 && n >= grid_warps * 64u) {
         const unsigned tail = grid_warps * 64u, per = 32u * R;                       // two one-ray batches per warp
         const unsigned g_rest0 = min(n_v, tail), p_rest0 = min(n_c, tail - g_rest0);
         const unsigned g_bulk = (n_v - g_rest0) / per * per, p_bulk = (n_c - p_rest0) / per * per;
         unsigned items = 0;
-        unsigned next = wf_cull_batches<R, BLOCK, true>(W, sc_, cur, p0, p0 + p_bulk, 0u, 0u, genC, 1, items, ITEM_NONE, budget, s_cullc, s_list);
+        unsigned next = wf_cull_batches<R, BLOCK, true, VIEWS>(W, sc_, cur, p0, p0 + p_bulk, 0u, 0u, genC, 1, items, ITEM_NONE, budget, s_cullc, s_list);
         items += p_bulk / per;
-        next = wf_cull_batches<R, BLOCK, false>(W, sc_, cur, 0u, g_bulk, n_g, p0, gen_base, 1, items, next, budget, s_cull, s_list);
+        next = wf_cull_batches<R, BLOCK, false, VIEWS>(W, sc_, cur, 0u, g_bulk, n_g, p0, gen_base, 1, items, next, budget, s_cull, s_list);
         items += g_bulk / per;
-        next = wf_cull_batches<1, BLOCK, true>(W, sc_, cur, p0 + p_bulk, p0 + n_c, 0u, 0u, genC, 1, items, next, budget, s_cullc, s_list);
+        next = wf_cull_batches<1, BLOCK, true, VIEWS>(W, sc_, cur, p0 + p_bulk, p0 + n_c, 0u, 0u, genC, 1, items, next, budget, s_cullc, s_list);
         items += (n_c - p_bulk + 31u) / 32u;
-        wf_cull_batches<1, BLOCK, false>(W, sc_, cur, g_bulk, n_v, n_g, p0, gen_base, 1, items, next, budget, s_cull, s_list);
+        wf_cull_batches<1, BLOCK, false, VIEWS>(W, sc_, cur, g_bulk, n_v, n_g, p0, gen_base, 1, items, next, budget, s_cull, s_list);
     } else {
         const unsigned b1 = (n + 31) / 32;
         int parts = 1;
@@ -770,14 +814,15 @@ __device__ __forceinline__ void wf_cull_body(const WaveParams& W, Scope sc_, int
             while (parts < 16 && b1 * (unsigned)parts * 2u <= grid_warps) parts *= 2;
         unsigned next = ITEM_NONE, items = 0;
         if (n_c) {
-            next = wf_cull_batches<1, BLOCK, true>(W, sc_, cur, p0, p0 + n_c, 0u, 0u, genC, parts, 0u, ITEM_NONE, budget, P.preloaded ? s_cullc : s_cull, s_list);
+            next = wf_cull_batches<1, BLOCK, true, VIEWS>(W, sc_, cur, p0, p0 + n_c, 0u, 0u, genC, parts, 0u, ITEM_NONE, budget, P.preloaded ? s_cullc : s_cull, s_list);
             items = (n_c + 31u) / 32u * (unsigned)parts;
         }
-        if (n_v) wf_cull_batches<1, BLOCK, false>(W, sc_, cur, 0u, n_v, n_g, p0, gen_base, parts, items, next, budget, s_cull, s_list);
+        if (n_v) wf_cull_batches<1, BLOCK, false, VIEWS>(W, sc_, cur, 0u, n_v, n_g, p0, gen_base, parts, items, next, budget, s_cull, s_list);
     }
 }
 
-template <int R, int BLOCK, int MINB>
+// VIEWS: instantiated for rt_render_views (false: single-camera renders, whose camera rays never leave P.cam)
+template <int R, int BLOCK, int MINB, bool VIEWS>
 __global__ void __launch_bounds__(BLOCK, MINB) wf_cull(const __grid_constant__ WaveParams W) {
     TraceScope trace(W.trace);
     const RenderParams& P = W.base;
@@ -796,7 +841,7 @@ __global__ void __launch_bounds__(BLOCK, MINB) wf_cull(const __grid_constant__ W
                 s_cullc[i] = Culler<R, BLOCK, true>::common_record(s_cull[i], P.cam.origin.x, P.cam.origin.y, P.cam.origin.z);
     }
     __syncthreads();
-    wf_cull_body<R, BLOCK>(W, grid_scope(), W.cur, n_g, n_p, gen_base, s_cull, s_cullc, s_list);
+    wf_cull_body<R, BLOCK, VIEWS>(W, grid_scope(), W.cur, n_g, n_p, gen_base, s_cull, s_cullc, s_list);
 }
 
 #include "rt_cull_tc.cuh"   // wf_cull_tc: the same cull on the tensor cores (tcgen05 / TMEM)
@@ -811,7 +856,7 @@ __device__ __forceinline__ unsigned wf_cand_region(const WaveParams& W, unsigned
 }
 
 // scp: the scene in the kernel's (grid-constant) parameter space — never the address of a local copy of the parameters
-template <bool GEN>
+template <bool GEN, bool VIEWS>
 __device__ __forceinline__ void wf_refine_body(const WaveParams& W, const DevScene* scp, Scope sc_, int cur) {
     const RenderParams& P = W.base;
     const unsigned npairs = min(W.st->npairs, W.pair_cap);
@@ -849,7 +894,7 @@ __device__ __forceinline__ void wf_refine_body(const WaveParams& W, const DevSce
                 uint32_t pixq = 0, smpq = 0, bq = 0;
                 if (__ldg(&P.sc.prim_type[pr.y]) == PRIM_MEDIUM) {   // its `rand` is keyed by the path (hitable.clj:529)
                     const uint32_t sd = __float_as_uint(qc[3 * (size_t)pr.x + 2].w);
-                    pixq = rng_pixel(P, __float_as_uint(b.w));
+                    pixq = rng_pixel<VIEWS>(P, __float_as_uint(b.w));
                     smpq = sd >> 8;
                     bq = (uint32_t)(P.max_depth - (int)(sd & 255u) + 1);
                 }
@@ -871,11 +916,11 @@ __device__ __forceinline__ void wf_refine_body(const WaveParams& W, const DevSce
     }
     if (lane == 0) W.cand_count[warp_id] = cnt;
 }
-template <bool GEN>
+template <bool GEN, bool VIEWS>
 __global__ void __launch_bounds__(256) wf_refine(const __grid_constant__ WaveParams W) {
     if (W.st->mode != MODE_RUN) return;
     TraceScope trace(W.trace);
-    wf_refine_body<GEN>(W, &W.base.sc, grid_scope(), W.cur);
+    wf_refine_body<GEN, VIEWS>(W, &W.base.sc, grid_scope(), W.cur);
 }
 
 // exact ties go to the lower caller index, the Hitlist rule (hitable.clj:17-26): candidates that own the final
@@ -919,7 +964,7 @@ __device__ __noinline__ void exact_closest_hit(const DevScene* sc, float ox, flo
 }
 
 // s_ctr: shared counters of the calling kernel (DC_COUNT slots, zeroed by the caller); returns samples generated
-template <bool GEN>
+template <bool GEN, bool VIEWS>
 __device__ __forceinline__ unsigned wf_shade_body(const WaveParams& W, const DevScene* scp, Scope sc_, int cur, unsigned* s_ctr) {
     const RenderParams& P = W.base;
     const unsigned n_g = W.st->cnt[cur][0], n_p = W.st->cnt[cur][1], n = n_g + n_p;
@@ -938,7 +983,7 @@ __device__ __forceinline__ unsigned wf_shade_body(const WaveParams& W, const Dev
             a = qc[3 * (size_t)idx]; b = qc[3 * (size_t)idx + 1]; c = qc[3 * (size_t)idx + 2];
             unsigned long long key = W.best_key[idx];
             const uint32_t slot = __float_as_uint(b.w), sd = __float_as_uint(c.w);   // slot: the pixel (a render) / the path (rt_trace_paths)
-            const uint32_t pix = rng_pixel(P, slot);
+            const uint32_t pix = rng_pixel<VIEWS>(P, slot);
             const uint32_t smp = sd >> 8;
             const int depth = (int)(sd & 255u);
             const uint32_t bounce = (uint32_t)(P.max_depth - depth + 1);
@@ -979,7 +1024,7 @@ __device__ __forceinline__ unsigned wf_shade_body(const WaveParams& W, const Dev
                 ScatterRng rng{P.key, pix, smp, bounce, nullptr, nullptr};
                 cont = shade_hit<GEN>(P.sc, scp, k, (float)td, o, d, tmv, depth > 0, rng, att, em, reason);
                 if (em.x != 0.f || em.y != 0.f || em.z != 0.f) {   // accum += atten * emitted (core.clj:32-34,37-39)
-                    float* dst = P.sum + (size_t)slot * 3;
+                    float* dst = P.sum + (size_t)frame_slot<VIEWS>(P, slot) * 3;
                     atomicAdd(dst + 0, c.x * em.x);
                     atomicAdd(dst + 1, c.y * em.y);
                     atomicAdd(dst + 2, c.z * em.z);
@@ -1012,7 +1057,7 @@ __device__ __forceinline__ unsigned wf_shade_body(const WaveParams& W, const Dev
     return 0u;
 }
 
-template <bool GEN>
+template <bool GEN, bool VIEWS>
 __global__ void __launch_bounds__(256, GEN ? 1 : 0) wf_shade(const __grid_constant__ WaveParams W) {
     if (W.st->mode != MODE_RUN) return;        // only this kernel's LAST CTA (below) or the tail ever change the mode
     TraceScope trace(W.trace);
@@ -1020,7 +1065,7 @@ __global__ void __launch_bounds__(256, GEN ? 1 : 0) wf_shade(const __grid_consta
     __shared__ unsigned s_ctr[DC_COUNT];
     if (threadIdx.x < DC_COUNT) s_ctr[threadIdx.x] = 0;
     __syncthreads();
-    wf_shade_body<GEN>(W, &W.base.sc, grid_scope(), W.cur, s_ctr);
+    wf_shade_body<GEN, VIEWS>(W, &W.base.sc, grid_scope(), W.cur, s_ctr);
     __syncthreads();
     if (threadIdx.x < DC_COUNT && s_ctr[threadIdx.x]) atomicAdd(&P.counters[threadIdx.x], (unsigned long long)s_ctr[threadIdx.x]);
     // The last CTA to finish hands out the next iteration's fresh work: the free slots of the other queue, as many as the
@@ -1132,7 +1177,7 @@ __device__ __forceinline__ BvhHit bvh_closest(const DevScene* sc, float ox, floa
 // one wavefront iteration's closest-hit search through the BVH: replaces wf_cull + wf_refine + wf_tiebreak.  One thread
 // per entry: load (or, for a fresh entry, generate) the ray, walk the tree, leave (t, key) in the closest-hit words for
 // wf_shade.  The direct spheres stay with wf_shade as in the brute-force path.
-template <bool GEN>
+template <bool GEN, bool VIEWS>
 __global__ void __launch_bounds__(128, GEN ? 1 : 0) wf_bvh(const __grid_constant__ WaveParams W) {
     if (W.st->mode != MODE_RUN) return;
     TraceScope trace(W.trace);
@@ -1150,7 +1195,7 @@ __global__ void __launch_bounds__(128, GEN ? 1 : 0) wf_bvh(const __grid_constant
         unsigned idx;
         if (v >= n_g) {
             idx = p0 + (v - n_g);
-            make_path(P, gen_base + (v - n_g), a, b, c);
+            make_path<VIEWS>(P, gen_base + (v - n_g), a, b, c);
             float4* q = qc + 3 * (size_t)idx;
             q[0] = a; q[1] = b; q[2] = c;
         } else {
@@ -1159,7 +1204,7 @@ __global__ void __launch_bounds__(128, GEN ? 1 : 0) wf_bvh(const __grid_constant
         }
         const uint32_t sd = __float_as_uint(c.w);
         const BvhHit H = bvh_closest<GEN>(&W.base.sc, a.x, a.y, a.z, b.x, b.y, b.z, a.w, 0.001, (double)FLT_MAX, true, P.key,
-                                          rng_pixel(P, __float_as_uint(b.w)), sd >> 8, (uint32_t)(P.max_depth - (int)(sd & 255u) + 1));
+                                          rng_pixel<VIEWS>(P, __float_as_uint(b.w)), sd >> 8, (uint32_t)(P.max_depth - (int)(sd & 255u) + 1));
         n_leaf += H.n_leaf; n_node += H.n_node;
         if (H.k >= 0) {
             W.best_t[idx] = (unsigned long long)__double_as_longlong(H.t);
@@ -1211,7 +1256,7 @@ __global__ void __launch_bounds__(128) trace_bvh_kernel(const __grid_constant__ 
 // key) — the merge rule of wf_refine + wf_tiebreak + wf_shade — and the shading runs on every lane of the group with
 // identical inputs (same Philox block); the group's first lane owns the side effects.  A group whose path has ended
 // claims the next one from the slice's shared counter.  Same arithmetic as the staged path: results equal bit for bit.
-template <bool GEN>
+template <bool GEN, bool VIEWS>
 __device__ __forceinline__ void wf_solo_paths(const WaveParams& W, const DevScene* scp, const float4* qc, unsigned n, unsigned* claim,
                                               const float4* s_cull, unsigned* s_ctr) {
     const RenderParams& P = W.base;
@@ -1230,7 +1275,7 @@ __device__ __forceinline__ void wf_solo_paths(const WaveParams& W, const DevScen
         if (!active && i < n) {
             a = qc[3 * (size_t)i]; b = qc[3 * (size_t)i + 1]; c = qc[3 * (size_t)i + 2];
             slot = __float_as_uint(b.w);
-            pix = rng_pixel(P, slot);
+            pix = rng_pixel<VIEWS>(P, slot);
             active = true;
         }
         if (!__any_sync(0xffffffffu, active)) break;
@@ -1291,7 +1336,7 @@ __device__ __forceinline__ void wf_solo_paths(const WaveParams& W, const DevScen
                 reason = TERM_NONE;
                 cont = shade_hit<GEN>(P.sc, scp, k, (float)td, o, d, tmv, depth > 0, rng, att, em, reason);
                 if (sub == 0u && (em.x != 0.f || em.y != 0.f || em.z != 0.f)) {   // accum += atten * emitted (core.clj:32-34,37-39)
-                    float* dst = P.sum + (size_t)slot * 3;
+                    float* dst = P.sum + (size_t)frame_slot<VIEWS>(P, slot) * 3;
                     atomicAdd(dst + 0, c.x * em.x);
                     atomicAdd(dst + 1, c.y * em.y);
                     atomicAdd(dst + 2, c.z * em.z);
@@ -1327,7 +1372,7 @@ constexpr int kPairsPerEntry = 8;       // pair buffer = 8 (ray, sphere) pairs p
 // TR: rays per thread of the tail's cull while a slice is still long (the first bounces after the hand-over, when a
 // slice holds thousands of paths): TR = 4 runs them like wf_cull does (4 independent chains per thread), the short-queue
 // forms (1 ray per thread, sphere list split across warps) take over as the slice shrinks.
-template <int BLOCK, bool GEN, int TR>
+template <int BLOCK, bool GEN, int TR, bool VIEWS>
 __global__ void __launch_bounds__(BLOCK, GEN ? 1 : 2) wf_tail(const __grid_constant__ WaveParams W) {
     const RenderParams& P = W.base;
     extern __shared__ float4 smem_f4[];
@@ -1384,20 +1429,20 @@ __global__ void __launch_bounds__(BLOCK, GEN ? 1 : 2) wf_tail(const __grid_const
             unsigned long long dt0 = global_timer_ns();
 #endif
             if (n <= W.tail_solo) {   // the thin end (or nothing): one warp per path, no more barriers (s_st.done: the claim counter)
-                if (n) wf_solo_paths<GEN>(L, &W.base.sc, cur ? L.queue[1] : L.queue[0], n, &s_st.done, s_cull, s_ctr);
+                if (n) wf_solo_paths<GEN, VIEWS>(L, &W.base.sc, cur ? L.queue[1] : L.queue[0], n, &s_st.done, s_cull, s_ctr);
 #ifdef RT_TAIL_DIAG
                 __syncthreads();
                 if (diag) printf("tail cta %u solo n %u: %llu ns\n", blockIdx.x, n, global_timer_ns() - dt0);
 #endif
                 break;
             }
-            wf_cull_body<TR, BLOCK>(L, solo, cur, n, 0u, 0ull, s_cull, nullptr, s_list);
+            wf_cull_body<TR, BLOCK, VIEWS>(L, solo, cur, n, 0u, 0ull, s_cull, nullptr, s_list);
             __syncthreads();
 #ifdef RT_TAIL_DIAG
             unsigned long long dt1 = global_timer_ns();
             const unsigned np_ = s_st.npairs;
 #endif
-            wf_refine_body<GEN>(L, &W.base.sc, solo, cur);
+            wf_refine_body<GEN, VIEWS>(L, &W.base.sc, solo, cur);
             __syncthreads();
 #ifdef RT_TAIL_DIAG
             unsigned long long dt2 = global_timer_ns();
@@ -1407,7 +1452,7 @@ __global__ void __launch_bounds__(BLOCK, GEN ? 1 : 2) wf_tail(const __grid_const
 #ifdef RT_TAIL_DIAG
             unsigned long long dt3 = global_timer_ns();
 #endif
-            wf_shade_body<GEN>(L, &W.base.sc, solo, cur, s_ctr);
+            wf_shade_body<GEN, VIEWS>(L, &W.base.sc, solo, cur, s_ctr);
 #ifdef RT_TAIL_DIAG
             __syncthreads();
             if (diag) printf("tail cta %u n %u pairs %u: cull %llu refine %llu tie %llu shade %llu ns\n", blockIdx.x, n, np_, dt1 - dt0, dt2 - dt1, dt3 - dt2, global_timer_ns() - dt3);
@@ -1465,8 +1510,8 @@ __device__ __noinline__ MegaShade mega_shade_one(const DevScene* scp, int k, flo
     return m;
 }
 
-template <int R, int BLOCK, int MINB, bool GEN>
-__global__ void __launch_bounds__(BLOCK, MINB) mega_kernel(const __grid_constant__ RenderParams P) {
+template <int R, int BLOCK, bool GEN, bool VIEWS>
+__device__ __forceinline__ void mega_body(const RenderParams& P) {
     extern __shared__ float4 smem_f4[];
     float4* s_cull = smem_f4;
     uint32_t* s_list = reinterpret_cast<uint32_t*>(smem_f4 + P.cull_cap);
@@ -1521,7 +1566,14 @@ __global__ void __launch_bounds__(BLOCK, MINB) mega_kernel(const __grid_constant
                         slot[r] = (uint32_t)w;
                     }
                     float3 o, d;
-                    generate_ray(P.cam, P.nx, P.ny, i, j, pix[r], smp[r], P.key, o, d, I.tm[r], nullptr);
+                    if (VIEWS && P.views && !P.path_pixel) {   // rt_render_views: as make_path
+                        const uint32_t v = view_of(P, slot[r]);
+                        pix[r] = slot[r] - v * P.view_px;
+                        const CameraRay cr = view_ray(P.views, v, P.nx, P.ny, i, j - (int)v * P.ny, pix[r], smp[r], P.key);
+                        o = cr.o; d = cr.d; I.tm[r] = cr.time;
+                    } else {
+                        generate_ray(P.cam, P.nx, P.ny, i, j, pix[r], smp[r], P.key, o, d, I.tm[r], nullptr);
+                    }
                     I.ox[r] = o.x; I.oy[r] = o.y; I.oz[r] = o.z;
                     I.dx[r] = d.x; I.dy[r] = d.y; I.dz[r] = d.z;
                     ar[r] = ag[r] = ab[r] = 1.0f;
@@ -1598,6 +1650,15 @@ __global__ void __launch_bounds__(BLOCK, MINB) mega_kernel(const __grid_constant
     atomicAdd(&s_ctr[DC_DIRECT], n_direct);
     __syncthreads();
     if (threadIdx.x < DC_COUNT && s_ctr[threadIdx.x]) atomicAdd(&P.counters[threadIdx.x], (unsigned long long)s_ctr[threadIdx.x]);
+}
+template <int R, int BLOCK, int MINB, bool GEN>
+__global__ void __launch_bounds__(BLOCK, MINB) mega_kernel(const __grid_constant__ RenderParams P) {
+    mega_body<R, BLOCK, GEN, false>(P);
+}
+// the megakernel of a batch of views (rt_render_views); the single-camera one above holds none of the batch code
+template <int R, int BLOCK, int MINB, bool GEN>
+__global__ void __launch_bounds__(BLOCK, MINB) mega_views_kernel(const __grid_constant__ RenderParams P) {
+    mega_body<R, BLOCK, GEN, true>(P);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1760,13 +1821,14 @@ struct ResolveParams {
     const float* peers[7];
     int n_peers;
     int nx, ny, nr;
+    int n_views;         // > 1: n_views stacked images of ny rows (rt_render_views), each flipped on its own
     uint8_t* rgb8;       // may be null
     float* mean;         // may be null: (float)(sum / nr), same layout as sum
     float* sum_out;      // may be null: reduced sum written back (multi-device)
 };
 __global__ void resolve_kernel(const ResolveParams P) {
-    int idx = blockIdx.x * blockDim.x + threadIdx.x;   // over nx*ny*3
-    int total = P.nx * P.ny * 3;
+    int idx = blockIdx.x * blockDim.x + threadIdx.x;   // over nx*ny*n_views*3
+    int total = P.nx * P.ny * 3 * (P.n_views > 1 ? P.n_views : 1);
     if (idx >= total) return;
     float s = P.sum[idx];
     for (int p = 0; p < P.n_peers; ++p) s += P.peers[p][idx];
@@ -1776,9 +1838,14 @@ __global__ void resolve_kernel(const ResolveParams P) {
     if (P.rgb8) {
         int ch = idx % 3, pixel = idx / 3;
         int i = pixel % P.nx, j = pixel / P.nx;
+        int row = P.ny - 1 - j;
+        if (P.n_views > 1) {   // row j of view v = j / ny lands on row ny - 1 - (j - v ny) of the view's image
+            const int v = j / P.ny;
+            row += 2 * v * P.ny;
+        }
         double y = sqrt(x) * 255.99;
         int v = (y != y) ? 0 : (int)fmin(255.99, y);   // (int NaN) = 0 on the JVM
-        P.rgb8[((size_t)(P.ny - 1 - j) * P.nx + i) * 3 + ch] = (uint8_t)v;
+        P.rgb8[((size_t)row * P.nx + i) * 3 + ch] = (uint8_t)v;
     }
 }
 

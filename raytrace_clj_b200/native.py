@@ -35,7 +35,7 @@ RT_TERM_LIGHT, RT_TERM_ABSORB, RT_TERM_DEPTH, RT_TERM_MISS = 1, 2, 3, 4
 RT_CTR_COUNT = 24
 COUNTER_NAMES = ["rays", "sphere_tests", "samples", "term_light", "term_absorb", "term_depth", "term_miss",
                  "kernel_ns", "candidates", "kernel_launches", "cull_ns", "refine_ns", "tiebreak_ns", "shade_ns",
-                 "direct_tests", "bvh_node_tests", "reduce_ns"]
+                 "direct_tests", "bvh_node_tests", "reduce_ns", "common_origin_rays"]
 
 # one logged bounce of rt_trace_paths (struct rt_path_bounce, 40 bytes)
 PATH_BOUNCE_DTYPE = np.dtype([("o", np.float32, 3), ("time", np.float32), ("d", np.float32, 3), ("hit_id", np.int32),
@@ -356,6 +356,34 @@ def marshal_camera(camera):
     raise UnsupportedSceneError(f"camera {type(camera).__name__} is not supported")
 
 
+def marshal_views(cameras):
+    """(cam_types int32[K], cams float32[K, 24]) for rt_render_views from a list of cameras: camera records
+    (camera.clj:8,35) or ``marshal_camera`` results ``(cam_type, float[24])``.  Pure host code: it checks the list's
+    shape and types and leaves the camera types themselves to the library, as ``rt_set_camera`` does."""
+    if isinstance(cameras, (str, bytes)) or not hasattr(cameras, "__len__"):
+        raise TypeError("cameras must be a list of cameras or of (cam_type, float[24]) pairs")
+    if len(cameras) == 0:
+        raise ValueError("cameras is empty: a batch renders at least one view")
+    types = np.empty(len(cameras), np.int32)
+    cams = np.empty((len(cameras), 24), np.float32)
+    for v, c in enumerate(cameras):
+        if isinstance(c, (cam.ThinLensCamera, cam.PinholeCamera)):
+            c = marshal_camera(c)
+        if not (isinstance(c, tuple) and len(c) == 2):
+            raise TypeError(f"view {v}: expected a camera or a (cam_type, float[24]) pair, got {type(c).__name__}")
+        t, f = c
+        if isinstance(t, (bool, np.bool_)) or not isinstance(t, (int, np.integer)):
+            raise TypeError(f"view {v}: the camera type must be an integer, got {type(t).__name__}")
+        f = np.asarray(f)
+        if f.shape != (24,):
+            raise ValueError(f"view {v}: a camera record has 24 floats, got shape {f.shape}")
+        if not np.issubdtype(f.dtype, np.floating):
+            raise TypeError(f"view {v}: a camera record holds floats, got {f.dtype}")
+        types[v] = t
+        cams[v] = f
+    return types, cams
+
+
 # ---------------------------------------------------------------------------------------------
 # ctypes binding
 # ---------------------------------------------------------------------------------------------
@@ -396,7 +424,8 @@ ABI_SYMBOLS = [
     "rt_render_accumulate_device", "rt_resolve_device", "rt_trace_primary", "rt_generate_rays", "rt_shade_batch",
     "rt_measure_fp32_peak", "rt_get_counters", "rt_reset_counters", "rt_set_profile", "rt_device_info", "rt_cull_check",
     "rt_set_scene_ex", "rt_trace_paths", "rt_set_accel", "rt_set_option", "rt_sample_device", "rt_host_alloc", "rt_host_free",
-    "rt_get_bvh", "rt_set_scene_device", "rt_get_scene_blob",
+    "rt_get_bvh", "rt_set_scene_device", "rt_get_scene_blob", "rt_render_views", "rt_render_views_accumulate_device",
+    "rt_resolve_views_device",
 ]
 
 _lib = None
@@ -445,6 +474,12 @@ def load_library():
     L.rt_get_bvh.argtypes = [C.c_void_p, C.c_int, _f32p, C.c_int64, C.POINTER(C.c_int64)]
     L.rt_set_scene_device.argtypes = [C.c_void_p, C.POINTER(_SceneDesc), C.c_void_p]
     L.rt_get_scene_blob.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)]
+    L.rt_render_views.argtypes = [C.c_void_p, C.c_int, _i32p, _f32p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_uint64,
+                                  C.c_int, _f32p, _u8p]
+    L.rt_render_views_accumulate_device.argtypes = [C.c_void_p, C.c_int, _i32p, _f32p, C.c_int, C.c_int, C.c_int, C.c_int,
+                                                    C.c_int, C.c_uint64, C.c_int, C.c_void_p, C.c_void_p, C.c_int]
+    L.rt_resolve_views_device.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
+                                          C.c_void_p, C.c_int]
     _lib = L
     return L
 
@@ -663,6 +698,35 @@ class Renderer:
         self._check(self.L.rt_render(self.h, nx, ny, nsamples, max_depth, C.c_uint64(seed), variant, _p(lin, _f32p),
                                      _p(img, _u8p)), "rt_render")
         return lin, img
+
+    def render_views(self, cameras, nx, ny, nsamples, max_depth=50, seed=1, variant=RT_VARIANT_WAVEFRONT, linear=True,
+                     rgb8=True):
+        """rt_render_views: K cameras (see ``marshal_views``) of the current scene in one call.  Returns (linear
+        [K,ny,nx,3] f32 | None, rgb8 [K,ny,nx,3] | None), every view in ``render``'s convention (linear: j = 0 at the
+        bottom; rgb8: row 0 at the top).  View v equals ``set_camera(camera v)`` + ``render`` up to the order of the
+        sample sums.  The context's camera is neither needed nor changed."""
+        types, cams = marshal_views(cameras)
+        k = len(types)
+        lin = np.empty((k, ny, nx, 3), np.float32) if linear else None
+        img = np.empty((k, ny, nx, 3), np.uint8) if rgb8 else None
+        self._check(self.L.rt_render_views(self.h, k, _p(types, _i32p), _p(cams, _f32p), nx, ny, nsamples, max_depth,
+                                           C.c_uint64(seed), variant, _p(lin, _f32p), _p(img, _u8p)), "rt_render_views")
+        return lin, img
+
+    def render_views_accumulate_device(self, cameras, nx, ny, sample_begin, sample_count, d_sum_ptr, max_depth=50, seed=1,
+                                       variant=RT_VARIANT_WAVEFRONT, stream=None, sync=True):
+        """d_sum (K*ny*nx*3 float32 on device 0, view v at offset v*nx*ny*3) += the views' samples [sample_begin,
+        sample_begin + sample_count)."""
+        types, cams = marshal_views(cameras)
+        self._check(self.L.rt_render_views_accumulate_device(
+            self.h, len(types), _p(types, _i32p), _p(cams, _f32p), nx, ny, sample_begin, sample_count, max_depth,
+            C.c_uint64(seed), variant, C.c_void_p(d_sum_ptr), C.c_void_p(stream or 0), 1 if sync else 0),
+            "rt_render_views_accumulate_device")
+
+    def resolve_views_device(self, n_views, nx, ny, nsamples_total, d_sum_ptr, d_rgb8_ptr, stream=None, sync=True):
+        self._check(self.L.rt_resolve_views_device(self.h, n_views, nx, ny, nsamples_total, C.c_void_p(d_sum_ptr),
+                                                   C.c_void_p(d_rgb8_ptr), C.c_void_p(stream or 0), 1 if sync else 0),
+                    "rt_resolve_views_device")
 
     def render_accumulate_device(self, nx, ny, sample_begin, sample_count, d_sum_ptr, row_offset=0, row_stride=1,
                                  max_depth=50, seed=1, variant=RT_VARIANT_WAVEFRONT, stream=None, sync=True):
